@@ -10,6 +10,8 @@ YOLOv9-E -> decode/NMS -> overlap filter (device) -> crop+resize -> Florence-2 g
 rank 0 with one NCCL gather.  `value` times it with the u8 screenshots already resident in HBM, `e2e` through the
 public API with host buffers (H2D of the screenshots and D2H of boxes/ids inside the timed region).
 Prints ONE JSON line on rank 0.
+
+  python bench.py ... --dump-outputs DIR    # also write what the last timed step returned as DIR/*.npy (see dump_outputs)
 """
 from __future__ import annotations
 
@@ -211,6 +213,38 @@ def _config(args, per_gpu_batch):
 
 
 # ------------------------------------------------------------------------------------------------ this repo
+SOURCES = ("box_ocr_content_ocr", "box_yolo_content_ocr", "box_yolo_content_yolo")
+
+
+def output_arrays(out):
+    """One step's results, ``[(elements, caption_ids)]`` per screenshot, as float64 arrays:
+    ``elements`` [N, 8] = screenshot, x0, y0, x1, y1 (ratios), interactivity, source (index into SOURCES), row of its
+    caption in ``caption_ids`` (-1: no caption); ``caption_ids`` [M, T] = greedy token ids, short rows padded with -1."""
+    elems, caps = [], []
+    for i, (el, ids) in enumerate(out):
+        first = len(caps)
+        caps.extend(ids.tolist())
+        row = first
+        for e in el:
+            src = SOURCES.index(e["source"])
+            elems.append([i, *e["bbox"], float(e["interactivity"]), src, row if src == 2 else -1])
+            row += src == 2
+        assert row == len(caps), "captioned elements and caption rows disagree"
+    width = max((len(r) for r in caps), default=0)
+    ids = np.full((len(caps), width), -1, np.float64)
+    for r, c in enumerate(caps):
+        ids[r, :len(c)] = c
+    return {"elements": np.asarray(elems, np.float64).reshape(-1, 8), "caption_ids": ids}
+
+
+def dump_outputs(arrays, out_dir):
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a)
+    log(f"outputs of the last timed step written to {d}: " + ", ".join(f"{k} {tuple(a.shape)}" for k, a in arrays.items()))
+
+
 def run_b200(args):
     rank, world, local = _dist()
     import torch.distributed as dist
@@ -230,6 +264,7 @@ def run_b200(args):
     sets = _inputs(rank, B)
     pipe = shard.GatherPipe(rank, world, dev, B, args.max_new_tokens, keep=False)   # one NCCL gather per step, on its own thread + stream
     stats = {"boxes": 0, "crops": 0, "n": 0}
+    last = [None]   # the results of the most recent step (--dump-outputs)
 
     def step(i, resident):
         imgs, ocr = sets[i % N_SETS]
@@ -239,6 +274,7 @@ def run_b200(args):
             io_["src"].copy_(dsets[i % N_SETS], non_blocking=True)      # device-to-device: input already in HBM
         out = parse_screenshots(imgs, model, cmp_, ocr, BOX_TRESHOLD=args.box_threshold, iou_threshold=0.7,
                                 max_new_tokens=args.max_new_tokens, timings=tm, _skip_h2d=resident)
+        last[0] = out
         stats["boxes"] += tm["n_boxes"]; stats["crops"] += tm["n_crops"]; stats["n"] += B
         pipe.submit(out)   # one gather of fixed-size padded records per step (SURVEY.md §8e); no-op at world 1
         return tm
@@ -264,6 +300,7 @@ def run_b200(args):
         res = (dsets[i % N_SETS] for i in range(n_steps)) if resident else None
         tm0 = dict(pp.timings)
         for out in pp.run(batches, res):
+            last[0] = out
             stats["n"] += B
             pipe.submit(out)
         stats["boxes"] += pp.timings["n_boxes"] - tm0["n_boxes"]
@@ -320,6 +357,7 @@ def run_b200(args):
         log("pipelined warm-up done")
     ms_res, _, launches, clocks, tms, st = timed("resident")
     log(f"resident leg: {ms_res / args.steps:.1f} ms/step")
+    outputs = output_arrays(last[0]) if args.dump_outputs else None   # the headline leg's last step, before later legs run
     ms_e2e, _, _, _, tms2, _ = timed("pinned")
     log(f"e2e leg: {ms_e2e / args.steps:.1f} ms/step")
     ms_pg = None
@@ -474,6 +512,8 @@ def run_b200(args):
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(args)
         print(json.dumps(line), flush=True)
+        if outputs is not None:
+            dump_outputs(outputs, args.dump_outputs)
     pipe.close()
     if world > 1:
         dist.barrier()
@@ -519,6 +559,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--with-768", action="store_true", help="B200 arm: also time the 768x768 caption mode (extra key caption_768)")
     ap.add_argument("--no-pipeline", action="store_true", help="one batch at a time (no detect/caption overlap across steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="B200 arm: write what the last timed step of the resident leg returned (rank 0's screenshots) as "
+                         "DIR/elements.npy and DIR/caption_ids.npy, float64; same arguments, same inputs")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

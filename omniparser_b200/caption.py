@@ -301,8 +301,11 @@ def find_tokenizer_dir(model_name_or_path=None, tokenizer_path=None) -> Optional
     if model_name_or_path:
         cands.append(Path(model_name_or_path).parent / "Florence-2-base")
     hub = Path(os.environ.get("HF_HOME", Path.home() / ".cache" / "huggingface")) / "hub" / "models--microsoft--Florence-2-base" / "snapshots"
-    if hub.is_dir():
-        cands.extend(sorted(hub.iterdir(), reverse=True))
+    try:
+        if hub.is_dir():
+            cands.extend(sorted(hub.iterdir(), reverse=True))
+    except PermissionError:   # a cache this user cannot read holds nothing for it
+        pass
     for c in cands:
         if (c / "tokenizer.json").is_file() or ((c / "vocab.json").is_file() and (c / "merges.txt").is_file()):
             return c

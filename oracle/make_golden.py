@@ -141,6 +141,151 @@ def real_goldens(ru, det, fl):
         print("wrote", out, len(raw.xyxy), "boxes,", ids.shape[0], "captions", flush=True)
 
 
+# What the CPU tests compare with the reference, beyond the parse goldens above: the reference's own functions run on the
+# tests' seeded inputs (the tests' input generators are imported from tests/, so inputs cannot drift apart).
+def _tests_module(name):
+    import importlib
+    import sys
+    tests = Path(__file__).resolve().parents[1] / "tests"
+    if str(tests) not in sys.path:
+        sys.path.insert(0, str(tests))
+    return importlib.import_module(name)
+
+
+def _write_json(name, gold):
+    out = GOLDEN / name
+    out.write_text(json.dumps(gold, separators=(",", ":")))
+    print("wrote", out, out.stat().st_size, "bytes", flush=True)
+
+
+def facade_calls_golden():
+    """ref:util/omniparser.py, unmodified, parses one 160x90 PNG with ``util.utils`` replaced by recorders: the functions
+    it calls and the arguments it passes them (tests/test_facade_cpu.py binds them to the drop-in's signatures)."""
+    import base64, inspect, io, sys, types
+    from .shims import REFERENCE
+    calls = []
+
+    def enc(v):
+        return {"pil_image": [v.size[0], v.size[1], v.mode]} if isinstance(v, Image.Image) else v
+
+    def rec(name, ret):
+        def f(*a, **k):
+            calls.append(dict(name=name, args=[enc(v) for v in a], kwargs={kk: enc(v) for kk, v in k.items()}))
+            return ret
+        return f
+
+    fake = types.ModuleType("util.utils")
+    fake.get_yolo_model = rec("get_yolo_model", "som")
+    fake.get_caption_model_processor = rec("get_caption_model_processor", {"model": "m", "processor": "p"})
+    fake.get_som_labeled_img = rec("get_som_labeled_img", ("b64", {"0": [0, 0, 1, 1]}, [{"type": "icon"}]))
+    fake.check_ocr_box = lambda image, **kw: ((["t"], [[1, 2, 30, 40]]), None)
+    pkg = types.ModuleType("util")
+    pkg.__path__ = [str(REFERENCE / "util")]
+    saved = {k: sys.modules.get(k) for k in ("util", "util.utils", "util.omniparser")}
+    sys.modules.update({"util": pkg, "util.utils": fake})
+    sys.modules.pop("util.omniparser", None)
+    try:
+        ro = __import__("util.omniparser", fromlist=["Omniparser"])
+        config = {"som_model_path": "weights/icon_detect_v3/model.pt", "caption_model_name": "florence2",
+                  "caption_model_path": "weights/icon_caption_florence", "BOX_TRESHOLD": 0.05}
+        op = ro.Omniparser(config)
+        buf = io.BytesIO()
+        Image.fromarray(np.zeros((90, 160, 3), np.uint8)).save(buf, format="PNG")
+        returned = op.parse(base64.b64encode(buf.getvalue()).decode("ascii"))
+        parse_parameters = list(inspect.signature(ro.Omniparser.parse).parameters)
+    finally:
+        for k, v in saved.items():
+            if v is None:
+                sys.modules.pop(k, None)
+            else:
+                sys.modules[k] = v
+    _write_json("reference_facade_calls.json", dict(config=config, calls=calls, returned=list(returned),
+                                                    parse_parameters=parse_parameters))
+
+
+def overlap_golden(ru):
+    """``remove_overlap_new`` (ref:util/utils.py:241-319) behind the ``int_box_area`` filters and the final sort of
+    ref:util/utils.py:437-451, on every case of tests/test_host_glue_cpu.py, stored in that test's compact encoding."""
+    import copy
+    T = _tests_module("test_host_glue_cpu")
+    whwh = torch.Tensor([T.W, T.H, T.W, T.H])
+    cases = {}
+    for kind, make, seeds in (("case", T._case, range(6)), ("dense", T._dense_case, range(12))):
+        for seed in seeds:
+            icons, ob, texts = make(seed)
+            ratio, oratio = icons.tolist(), (torch.tensor(ob) / whwh).tolist()
+            for thr in T.THRESHOLDS:
+                ocr_elem = [{'type': 'text', 'bbox': box, 'interactivity': False, 'content': txt, 'source': 'box_ocr_content_ocr'}
+                            for box, txt in zip(oratio, texts) if ru.int_box_area(box, T.W, T.H) > 0]
+                xyxy_elem = [{'type': 'icon', 'bbox': box, 'interactivity': True, 'content': None} for box in ratio
+                             if ru.int_box_area(box, T.W, T.H) > 0]
+                ref = ru.remove_overlap_new(boxes=xyxy_elem, iou_threshold=thr, ocr_bbox=copy.deepcopy(ocr_elem))
+                ref = sorted(ref, key=lambda x: x['content'] is None)
+                enc = []
+                for e in ref:
+                    if e["source"] == "box_ocr_content_ocr":
+                        enc.append(["o", next(k for k in range(len(oratio)) if oratio[k] == e["bbox"] and texts[k] == e["content"])])
+                    else:
+                        enc.append(["i", ratio.index(e["bbox"]), e["content"]])
+                assert T.decode_elements(enc, ratio, oratio, texts) == ref
+                cases[T.case_key(kind, seed, thr)] = enc
+    _write_json("reference_remove_overlap_new.json", cases)
+
+
+def predict_golden(ry, path):
+    """``YOLOv9Detector.predict`` (ref:util/yolov9.py:115-136) on the TorchScript stand-in, tests/test_oracle_cpu.py's case."""
+    T = _tests_module("test_oracle_cpu")
+    det = ry.YOLOv9Detector(model_path=path, device="cpu")
+    ref = det.predict(Image.fromarray(synth.screenshot(T.PREDICT_SEED)), conf=T.PREDICT_CONF, iou=T.PREDICT_IOU)[0].boxes
+    _write_json("reference_yolov9_predict.json", dict(seed=T.PREDICT_SEED, conf=T.PREDICT_CONF, iou=T.PREDICT_IOU,
+                                                      xyxy=ref.xyxy.tolist(), scores=ref.conf.tolist()))
+
+
+def check_ocr_box_golden(ru):
+    """``check_ocr_box`` (ref:util/utils.py:514-549) driven by tests/test_serving_cpu.py's fake OCR engines; ``repr`` of the
+    result, so that tuples, lists and number types are pinned too."""
+    T = _tests_module("test_serving_cpu")
+    old_r, old_p = ru.reader, ru.paddle_ocr
+    ru.reader, ru.paddle_ocr = T._Reader(), T._Paddle()
+    try:
+        img = T.ocr_golden_image()
+        calls = [dict(kwargs=kw, repr=repr(ru.check_ocr_box(img, display_img=False, goal_filtering=None, **kw)))
+                 for kw in T.OCR_KWARGS]
+    finally:
+        ru.reader, ru.paddle_ocr = old_r, old_p
+    _write_json("reference_check_ocr_box.json", calls)
+
+
+def annotate_golden(ru):
+    """``annotate`` (ref:util/utils.py:336-366, util/box_annotator.py) on tests/test_overlay_cpu.py's layouts: sha256 of
+    the annotated frame and the label coordinates, in one .npz."""
+    import hashlib
+    from torchvision.ops import box_convert
+    T = _tests_module("test_overlay_cpu")
+    arrays = {}
+    for seed, n, (w, h), cfg in T.LAYOUTS:
+        for crowded in (False, True):
+            img = synth.screenshot(seed, w, h)
+            boxes = T._layout(seed, n, w, h, crowded)
+            t = box_convert(torch.tensor(boxes).reshape(-1, 4), "xyxy", "cxcywh")
+            frame, coords = ru.annotate(image_source=img, boxes=t, logits=None, phrases=list(range(n)), **cfg)
+            key = T.layout_key(seed, crowded)
+            arrays[key + "_sha256"] = np.array(hashlib.sha256(frame.tobytes()).hexdigest())
+            arrays[key + "_shape"] = np.array(frame.shape, np.int64)
+            arrays[key + "_coords"] = np.array([coords[str(i)] for i in range(n)], np.float32).reshape(n, 4)
+    out = GOLDEN / "reference_annotate_layouts.npz"
+    np.savez_compressed(out, **arrays)
+    print("wrote", out, out.stat().st_size, "bytes", flush=True)
+
+
+def reference_call_goldens(ru, ry, path):
+    facade_calls_golden()
+    overlap_golden(ru)
+    predict_golden(ry, path)
+    check_ocr_box_golden(ru)
+    annotate_golden(ru)
+
+
 def main():
     import sys
     ru, ry = import_reference()
@@ -152,6 +297,9 @@ def main():
     fl = FS.florence_standin(0)
     if "real" in sys.argv[1:]:          # python -m oracle.make_golden real  -> only the real-image goldens
         real_goldens(ru, det, fl)
+        return
+    if "calls" in sys.argv[1:]:         # python -m oracle.make_golden calls -> only the reference-call goldens
+        reference_call_goldens(ru, ry, path)
         return
     for case in CASES:
         w, h = case["size"]
@@ -174,6 +322,7 @@ def main():
         print("wrote", out, len(raw.xyxy), "boxes,", ids.shape[0], "captions")
     facade_golden(path, fl)
     real_goldens(ru, det, fl)
+    reference_call_goldens(ru, ry, path)
 
 
 if __name__ == "__main__":

@@ -1,52 +1,37 @@
 """CPU: the reference facade (ref:util/omniparser.py:7-32), UNMODIFIED, calls the three hot functions with arguments that
 bind to the drop-in's signatures -- i.e. swapping ``util.utils`` for ``omniparser_b200.utils`` in its import line is the whole
-integration.  Runs where /root/reference exists; tests/test_boundary_gpu.py runs the swapped facade for real on the GPU."""
-import base64
+integration.  The calls are the ones the reference file made when it parsed a 160x90 PNG with recorders in place of
+``util.utils`` (tests/golden/reference_facade_calls.json, written by oracle/make_golden.py); tests/test_boundary_gpu.py runs
+the swapped facade for real on the GPU."""
 import inspect
-import io
-import sys
-import types
+import json
+from pathlib import Path
 
-import numpy as np
-import pytest
 from PIL import Image
 
 from omniparser_b200 import utils as B
-from oracle.shims import REFERENCE, reference_available
+
+GOLD = Path(__file__).resolve().parent / "golden"
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present")
-def test_reference_facade_binds_to_the_drop_in_signatures(monkeypatch):
+def _decode(v):
+    if isinstance(v, dict) and set(v) == {"pil_image"}:
+        w, h, mode = v["pil_image"]
+        return Image.new(mode, (w, h))
+    return v
+
+
+def test_reference_facade_binds_to_the_drop_in_signatures():
+    g = json.loads((GOLD / "reference_facade_calls.json").read_text())
+    drop_in = {"get_yolo_model": B.get_yolo_model, "get_caption_model_processor": B.get_caption_model_processor,
+               "get_som_labeled_img": B.get_som_labeled_img}
     calls = []
-
-    def bound(fn, ret):
-        sig = inspect.signature(fn)
-
-        def f(*a, **k):
-            ba = sig.bind(*a, **k)          # TypeError here = the reference passes something the drop-in does not accept
-            calls.append((fn.__name__, dict(ba.arguments)))
-            return ret
-        return f
-
-    fake = types.ModuleType("util.utils")
-    fake.get_yolo_model = bound(B.get_yolo_model, "som")
-    fake.get_caption_model_processor = bound(B.get_caption_model_processor, {"model": "m", "processor": "p"})
-    fake.get_som_labeled_img = bound(B.get_som_labeled_img, ("b64", {"0": [0, 0, 1, 1]}, [{"type": "icon"}]))
-    fake.check_ocr_box = lambda image, **kw: ((["t"], [[1, 2, 30, 40]]), None)
-    pkg = types.ModuleType("util")
-    pkg.__path__ = [str(REFERENCE / "util")]
-    monkeypatch.setitem(sys.modules, "util", pkg)
-    monkeypatch.setitem(sys.modules, "util.utils", fake)
-    monkeypatch.delitem(sys.modules, "util.omniparser", raising=False)
-    monkeypatch.syspath_prepend(str(REFERENCE))
-    import importlib
-    ro = importlib.import_module("util.omniparser")            # the reference file itself, byte for byte
-    op = ro.Omniparser({"som_model_path": "weights/icon_detect_v3/model.pt", "caption_model_name": "florence2",
-                        "caption_model_path": "weights/icon_caption_florence", "BOX_TRESHOLD": 0.05})
-    buf = io.BytesIO()
-    Image.fromarray(np.zeros((90, 160, 3), np.uint8)).save(buf, format="PNG")
-    out = op.parse(base64.b64encode(buf.getvalue()).decode("ascii"))
-    assert out == ("b64", [{"type": "icon"}])
+    for c in g["calls"]:
+        sig = inspect.signature(drop_in[c["name"]])
+        # TypeError here = the reference passes something the drop-in does not accept
+        ba = sig.bind(*[_decode(v) for v in c["args"]], **{k: _decode(v) for k, v in c["kwargs"].items()})
+        calls.append((c["name"], dict(ba.arguments)))
+    assert g["returned"] == ["b64", [{"type": "icon"}]]
     names = [c[0] for c in calls]
     assert names == ["get_yolo_model", "get_caption_model_processor", "get_som_labeled_img"]
     kw = calls[2][1]
@@ -54,4 +39,4 @@ def test_reference_facade_binds_to_the_drop_in_signatures(monkeypatch):
     assert set(kw["draw_bbox_config"]) == {"text_scale", "text_thickness", "text_padding", "thickness"}
     # the drop-in's own facade is the same file after the import swap: same public surface
     from omniparser_b200.omniparser import Omniparser
-    assert list(inspect.signature(Omniparser.parse).parameters) == list(inspect.signature(ro.Omniparser.parse).parameters)
+    assert list(inspect.signature(Omniparser.parse).parameters) == g["parse_parameters"]

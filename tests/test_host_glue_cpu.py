@@ -1,6 +1,8 @@
-"""CPU: host list logic (overlap filter, element construction) of the product vs the unmodified reference functions
-(when /root/reference exists) and vs the oracle's independent restatement."""
-import copy
+"""CPU: host list logic (overlap filter, element construction) of the product vs what the unmodified reference functions
+returned on the same cases (tests/golden/reference_remove_overlap_new.json, written by oracle/make_golden.py) and vs the
+oracle's independent restatement."""
+import json
+from pathlib import Path
 
 import numpy as np
 import pytest
@@ -8,9 +10,32 @@ import torch
 
 from omniparser_b200 import host_glue
 from oracle import pipeline_cpu
-from oracle.shims import reference_available
 
 W, H = 1920, 1080
+THRESHOLDS = (0.7, 0.9)
+GOLD = Path(__file__).resolve().parent / "golden"
+
+
+def case_key(kind, seed, thr):
+    return f"{kind}{seed}_iou{thr}"
+
+
+def decode_elements(enc, icons, oboxes, texts):
+    """The reference's element list from its golden encoding: ["o", k] is the OCR element of input box k, ["i", j, content]
+    the icon element of input box j (the encoding is checked to round-trip when the golden is written)."""
+    out = []
+    for e in enc:
+        if e[0] == "o":
+            out.append({'type': 'text', 'bbox': oboxes[e[1]], 'interactivity': False, 'content': texts[e[1]], 'source': 'box_ocr_content_ocr'})
+        else:
+            out.append({'type': 'icon', 'bbox': icons[e[1]], 'interactivity': True, 'content': e[2],
+                        'source': 'box_yolo_content_ocr' if e[2] is not None else 'box_yolo_content_yolo'})
+    return out
+
+
+def reference_elements(kind, seed, thr, icons, oboxes, texts):
+    gold = json.loads((GOLD / "reference_remove_overlap_new.json").read_text())
+    return decode_elements(gold[case_key(kind, seed, thr)], icons, oboxes, texts)
 
 
 def _case(seed, n_icon=70, n_ocr=20):
@@ -49,22 +74,14 @@ def test_build_elements_matches_oracle_restatement(seed, thr):
     assert start == next((i for i, e in enumerate(a) if e["content"] is None), -1)
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not on this machine")
 @pytest.mark.parametrize("seed", range(6))
 def test_build_elements_matches_reference(seed):
-    from oracle.shims import import_reference
-    ru, _ = import_reference()
     icons, ob, texts = _case(seed)
     whwh = torch.Tensor([W, H, W, H])
-    for thr in (0.7, 0.9):
-        # ref:util/utils.py:437-451 verbatim call sequence
+    for thr in THRESHOLDS:
+        # the reference ran ref:util/utils.py:437-451 verbatim on these inputs
         ocr_bbox = (torch.tensor(ob) / whwh).tolist()
-        ocr_elem = [{'type': 'text', 'bbox': box, 'interactivity': False, 'content': txt, 'source': 'box_ocr_content_ocr'}
-                    for box, txt in zip(ocr_bbox, texts) if ru.int_box_area(box, W, H) > 0]
-        xyxy_elem = [{'type': 'icon', 'bbox': box, 'interactivity': True, 'content': None} for box in icons.tolist()
-                     if ru.int_box_area(box, W, H) > 0]
-        ref = ru.remove_overlap_new(boxes=xyxy_elem, iou_threshold=thr, ocr_bbox=copy.deepcopy(ocr_elem))
-        ref = sorted(ref, key=lambda x: x['content'] is None)
+        ref = reference_elements("case", seed, thr, icons.tolist(), ocr_bbox, texts)
         got, _ = host_glue.build_elements(icons.tolist(), ocr_bbox, texts, W, H, thr)
         assert got == ref
 
@@ -100,20 +117,12 @@ def test_dense_overlaps_fast_equals_loops_and_reference(seed):
     icons, ob, texts = _dense_case(seed)
     whwh = torch.Tensor([W, H, W, H])
     oratio = (torch.tensor(ob) / whwh).tolist()
-    for thr in (0.7, 0.9):
+    for thr in THRESHOLDS:
         fast, _ = host_glue.build_elements(icons.tolist(), oratio, texts, W, H, thr)
         slow, _ = host_glue.build_elements(icons.tolist(), oratio, texts, W, H, thr, fast=False)
         assert fast == slow
         assert any(e["source"] == "box_yolo_content_ocr" for e in fast), "case does not exercise label collection"
-        if reference_available():
-            from oracle.shims import import_reference
-            ru, _ = import_reference()
-            ocr_elem = [{'type': 'text', 'bbox': box, 'interactivity': False, 'content': txt, 'source': 'box_ocr_content_ocr'}
-                        for box, txt in zip(oratio, texts) if ru.int_box_area(box, W, H) > 0]
-            xyxy_elem = [{'type': 'icon', 'bbox': box, 'interactivity': True, 'content': None} for box in icons.tolist()
-                         if ru.int_box_area(box, W, H) > 0]
-            ref = ru.remove_overlap_new(boxes=xyxy_elem, iou_threshold=thr, ocr_bbox=copy.deepcopy(ocr_elem))
-            assert fast == sorted(ref, key=lambda x: x['content'] is None)
+        assert fast == reference_elements("dense", seed, thr, icons.tolist(), oratio, texts)
 
 
 # ---------------------------------------------------------------------------------------------- device-filter contract

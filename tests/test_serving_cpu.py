@@ -1,11 +1,14 @@
 """CPU: the two "next" rows around the hot path that are pure host logic --
 * §8f-3 ``omniparser_b200.ocr.check_ocr_box`` (the reference's OCR pre-step adapter, ref:util/utils.py:498-549) against fake
-  engines and, where /root/reference exists, against the UNMODIFIED reference function driven by the same fake engines;
+  engines and against what the UNMODIFIED reference function returned when driven by the same fake engines
+  (tests/golden/reference_check_ocr_box.json, written by oracle/make_golden.py);
 * §8f-4 ``omniparser_b200.server.DynamicBatcher`` / ``create_app`` (cross-request batching behind the reference server's wire
   format, ref:omnitool/omniparserserver/omniparserserver.py:37-48): grouping by key, size and deadline triggers, order,
   error delivery, concurrency."""
+import json
 import threading
 import time
+from pathlib import Path
 
 import numpy as np
 import pytest
@@ -13,8 +16,8 @@ from PIL import Image
 
 from omniparser_b200 import ocr as OCR
 from omniparser_b200.server import DynamicBatcher
-from oracle.shims import reference_available
 
+GOLD = Path(__file__).resolve().parent / "golden"
 QUADS = [([[10.7, 20.2], [110.1, 20.2], [110.1, 44.9], [10.7, 44.9]], "File", 0.93),
          ([[300, 400], [420, 400], [420, 431], [300, 431]], "Edit view", 0.41),
          ([[5.5, 600.5], [64.4, 600.5], [64.4, 630.0], [5.5, 630.0]], "x", 0.77)]
@@ -67,21 +70,22 @@ def test_check_ocr_box_formats(engines, mode, tmp_path):
     assert OCR.get_xywh_yolo([3.9, 4.2, 10.1, 20.9]) == (3, 4, 6, 16)
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not on this machine")
+OCR_KWARGS = [dict(output_bb_format="xyxy"), dict(output_bb_format="xywh"), dict(output_bb_format="xyxy", use_paddleocr=True),
+              dict(output_bb_format="xyxy", use_paddleocr=True, easyocr_args={"text_threshold": 0.8}),
+              dict(output_bb_format="xyxy", easyocr_args={"text_threshold": 0.8})]
+
+
+def ocr_golden_image():
+    return Image.fromarray(np.zeros((700, 500, 4), np.uint8), "RGBA")
+
+
 def test_check_ocr_box_equals_unmodified_reference(engines):
-    from oracle.shims import import_reference
-    ru, _ = import_reference()
-    reader, paddle = engines
-    old_r, old_p = ru.reader, ru.paddle_ocr
-    ru.reader, ru.paddle_ocr = reader, paddle
-    try:
-        img = Image.fromarray(np.zeros((700, 500, 4), np.uint8), "RGBA")
-        for kw in (dict(output_bb_format="xyxy"), dict(output_bb_format="xywh"), dict(output_bb_format="xyxy", use_paddleocr=True),
-                   dict(output_bb_format="xyxy", use_paddleocr=True, easyocr_args={"text_threshold": 0.8}),
-                   dict(output_bb_format="xyxy", easyocr_args={"text_threshold": 0.8})):
-            assert OCR.check_ocr_box(img, display_img=False, goal_filtering=None, **kw) == ru.check_ocr_box(img, display_img=False, goal_filtering=None, **kw)
-    finally:
-        ru.reader, ru.paddle_ocr = old_r, old_p
+    """Same engines, same arguments: the same ``repr`` as the reference's result (tuples vs lists and number types included)."""
+    gold = json.loads((GOLD / "reference_check_ocr_box.json").read_text())
+    assert [g["kwargs"] for g in gold] == OCR_KWARGS
+    img = ocr_golden_image()
+    for g in gold:
+        assert repr(OCR.check_ocr_box(img, display_img=False, goal_filtering=None, **g["kwargs"])) == g["repr"]
 
 
 def test_missing_engine_raises_clearly(monkeypatch):
