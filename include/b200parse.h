@@ -128,14 +128,6 @@ int b2p_crop_resize(const unsigned char* imgs, const int* img_hw, const long lon
 /* ---- Florence-2 (HF generate, ref:util/utils.py:125): non-GEMM kernels; `split` selects the fp16x3 layout ---- */
 int b2p_layernorm(const float* x, long long ldx, const float* gamma, const float* beta, float eps, int T, int C,
                   void* out16, long long ld16, float* out32, long long ld32, int split, b2p_stream_t stream);
-/* LayerNorm(A * B^T + bias + residual) for the decoder's split-K GEMMs that feed a LayerNorm (hf:models/bart/modeling_bart.py:
- * 312-391: out-proj / cross out-proj / fc2 + residual + layer norm): the GEMM parks its raw partial tiles, one more kernel sums
- * the k slices, adds bias + residual and normalises.  flags as b2p_gemm (bit 3: fp16x3 operands, bit 2: out16 as [hi | lo]). */
-int b2p_gemm_ln(const void* A, long long lda, const void* B, int M, int N, int K, const float* bias, const float* residual,
-                long long ldr, const float* gamma, const float* beta, float eps, void* out16, long long ld16, float* out32,
-                long long ld32, int flags, b2p_stream_t stream);
-int b2p_dwconv3x3_res(const float* x, int B, int H, int W, int C, const float* w9c, const float* bias, float* y,
-                      b2p_stream_t stream);
 int b2p_dwconv_ln(const float* x, int B, int H, int W, int C, const float* w9c, const float* bias, float* y,
                   const float* gamma, const float* beta, float eps, void* out16, int split, b2p_stream_t stream);
 int b2p_window_attn(const float* qkv, const float* qkv_bias, int B, int H, int W, int C, int heads, int win, void* out,

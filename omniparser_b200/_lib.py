@@ -47,8 +47,6 @@ PROTOTYPES = {
     "b2p_overlap_filter": (i32, [vp, vp, i32, i32, vp, vp, vp, vp, i32, f64, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "b2p_crop_resize": (i32, [vp, vp, vp, vp, vp, i32, i32, vp, vp, vp]),
     "b2p_layernorm": (i32, [vp, i64, vp, vp, f32, i32, i32, vp, i64, vp, i64, i32, vp]),
-    "b2p_gemm_ln": (i32, [vp, i64, vp, i32, i32, i32, vp, vp, i64, vp, vp, f32, vp, i64, vp, i64, i32, vp]),
-    "b2p_dwconv3x3_res": (i32, [vp, i32, i32, i32, i32, vp, vp, vp, vp]),
     "b2p_dwconv_ln": (i32, [vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, f32, vp, i32, vp]),
     "b2p_window_attn": (i32, [vp, vp, i32, i32, i32, i32, i32, i32, vp, i32, vp]),
     "b2p_channel_attn": (i32, [vp, i32, i32, i32, i32, vp, i32, vp]),

@@ -50,7 +50,7 @@ const char* b2p_last_error(void) {
 
 long long b2p_launch_count(void) { return g_launches.load(); }
 
-int b2p_abi_version(void) { return 2; }
+int b2p_abi_version(void) { return 3; }
 
 // Debugging aid (B2P_TRACE=1): per-CTA phase timestamps of the traced GEMM launches, see gemm_tcgen05.cu::trace_read.
 int b2p_trace_read(unsigned long long* stamps, int* meta, int max_launches) { return trace_read(stamps, meta, max_launches); }

@@ -18,10 +18,6 @@ void count_launch(int n = 1);     // bumps the kernel-launch counter read by b2p
     b2p::count_launch();                                            \
   } while (0)
 
-// Where a park-only GEMM left its partial accumulators: element (tile, slice s, row r, column c) at
-// ws[((tile * ksplit + s) * 128 + r) * bn + c], tile = mt_fast ? nt * m_tiles + mt : mt * n_tiles + nt.
-struct ParkInfo { float* ws; int bn, ksplit, n_tiles, m_tiles, mt_fast; };
-
 // Descriptor of one dense contraction for gemm_launch().
 struct ConvGemm {
   int mode;            // 0 = GEMM rows, 1 = conv3x3 s1 p1, 2 = conv3x3 s2 p1   (NHWC)
@@ -48,9 +44,6 @@ struct ConvGemm {
   long long lo_a;      // A: lo half at column lo_a + k            (default K / Cin)
   long long lo_out;    // split_out: lo half at column lo_out + n  (default N)
   long long lo_res;    // fp16 residual is a hi/lo pair, lo at column lo_res + n (default: residual has no lo half)
-  int park;            // 1 = park-only (mode 0): raw fp32 accumulators of every (tile, k slice) stay in the split-K workspace; no
-                       // bias / activation / residual / store -- the caller runs the consumer kernel (florence_ops.cu: b2p_gemm_ln)
-  ParkInfo* park_info; // filled when park != 0
 };
 
 int gemm_launch(const ConvGemm& d, cudaStream_t st);

@@ -72,70 +72,6 @@ __global__ void layernorm_kernel(const float* __restrict__ x, long long ldx, con
   }
 }
 
-// Split-K reduction + bias + residual + LayerNorm in one pass over the partial tiles a park-only GEMM left in the split-K
-// workspace (gemm_tcgen05.cu, GemmArgs::park): the decoder's out-proj / cross out-proj / fc2 GEMMs (N = 768, M = crops) are
-// split-K launches followed by a LayerNorm; inside the GEMM the slices had to wait for each other and re-read the partials
-// (5.8 of 10.8 us), and the LayerNorm was one more 4 us launch.  One warp per row.  Same arithmetic in the same order as
-// the GEMM epilogue (slices in order, + bias, + residual) and layernorm_kernel => bit-identical results.
-__global__ void splitk_ln_kernel(ParkInfo pk, int M, int N, const float* __restrict__ bias, const float* __restrict__ res, long long ldr,
-                                 const float* __restrict__ g, const float* __restrict__ b, float eps, __half* __restrict__ o16,
-                                 long long ld16, float* __restrict__ o32, long long ld32, int split) {
-  pdl_wait();
-  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  const int lane = threadIdx.x & 31;
-  if (row >= M) return;
-  const int mt = row >> 7, r = row & 127;
-  const int C4 = N >> 2;
-  const size_t sl_stride = size_t(128) * pk.bn;     // floats between consecutive k slices of a tile
-  float4 v[8];   // N <= 1024
-  float s = 0.f;
-  int n = 0;
-  for (int c = lane; c < C4; c += 32, ++n) {
-    const int col = 4 * c;
-    const int nt = col / pk.bn, cc = col - nt * pk.bn;
-    const int tile = pk.mt_fast ? nt * pk.m_tiles + mt : mt * pk.n_tiles + nt;
-    const float* p = pk.ws + (size_t(tile) * pk.ksplit * 128 + r) * pk.bn + cc;
-    float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-    int sidx = 0;
-    for (; sidx + 2 <= pk.ksplit; sidx += 2) {       // two slices in flight; adds in slice order
-      const float4 t0 = __ldcg(reinterpret_cast<const float4*>(p + size_t(sidx) * sl_stride));
-      const float4 t1 = __ldcg(reinterpret_cast<const float4*>(p + size_t(sidx + 1) * sl_stride));
-      a.x += t0.x; a.y += t0.y; a.z += t0.z; a.w += t0.w;
-      a.x += t1.x; a.y += t1.y; a.z += t1.z; a.w += t1.w;
-    }
-    if (sidx < pk.ksplit) {
-      const float4 t0 = __ldcg(reinterpret_cast<const float4*>(p + size_t(sidx) * sl_stride));
-      a.x += t0.x; a.y += t0.y; a.z += t0.z; a.w += t0.w;
-    }
-    if (bias) {
-      const float4 bb = reinterpret_cast<const float4*>(bias)[c];
-      a.x += bb.x; a.y += bb.y; a.z += bb.z; a.w += bb.w;
-    }
-    if (res) {
-      const float4 rr = reinterpret_cast<const float4*>(res + (long long)row * ldr)[c];
-      a.x += rr.x; a.y += rr.y; a.z += rr.z; a.w += rr.w;
-    }
-    v[n] = a;
-    s += (a.x + a.y) + (a.z + a.w);
-  }
-  const float mean = warp_sum(s) / float(N);
-  float q = 0.f;
-  for (int i = 0; i < n; ++i) {
-    const float dx = v[i].x - mean, dy = v[i].y - mean, dz = v[i].z - mean, dw = v[i].w - mean;
-    q += (dx * dx + dy * dy) + (dz * dz + dw * dw);
-  }
-  const float rstd = rsqrtf(warp_sum(q) / float(N) + eps);
-  n = 0;
-  for (int c = lane; c < C4; c += 32, ++n) {
-    const float4 gg = reinterpret_cast<const float4*>(g)[c], bb = reinterpret_cast<const float4*>(b)[c];
-    float4 y;
-    y.x = (v[n].x - mean) * rstd * gg.x + bb.x; y.y = (v[n].y - mean) * rstd * gg.y + bb.y;
-    y.z = (v[n].z - mean) * rstd * gg.z + bb.z; y.w = (v[n].w - mean) * rstd * gg.w + bb.w;
-    if (o16) store_act4(o16 + (long long)row * ld16, 4 * c, split, y);
-    if (o32) reinterpret_cast<float4*>(o32 + (long long)row * ld32)[c] = y;
-  }
-}
-
 // Fused DaViT pre-block: y = dwconv3x3(x) + bias + x (fp32, the new residual stream) and h = LayerNorm(y) as the next
 // GEMM operand.  One warp per token; channels in float4 lanes (C <= 1024).
 __global__ void dwconv_ln_kernel(const float* __restrict__ x, int B, int H, int W, int C, const float* __restrict__ w9c,
@@ -189,109 +125,16 @@ __global__ void dwconv_ln_kernel(const float* __restrict__ x, int B, int H, int 
   }
 }
 
-// Tiled variant (split bit 1; the default since it was validated on the B200 in round 2, B2P_NO_DWCONV_TILE=1 disables it): one CTA
-// per image stages the whole H x W x C map in shared memory once, so the nine taps read smem instead of re-reading L2 nine
-// times (the per-token kernel above moves ~36 B per element through L2: 24 us per launch where HBM needs 5).  Same
-// arithmetic in the same order as dwconv_ln_kernel => bit-identical outputs (tests/test_ops_gpu.py, gated).
-__global__ void dwconv_ln_tile_kernel(const float* __restrict__ x, int H, int W, int C, const float* __restrict__ w9c,
-                                      const float* __restrict__ bias, float* __restrict__ y, const float* __restrict__ g,
-                                      const float* __restrict__ bt, float eps, __half* __restrict__ o16, int split) {
-  pdl_wait();
-  extern __shared__ float4 xs4[];   // [H*W][C/4]
-  const int HW = H * W, C4 = C >> 2;
-  const long long tok0 = (long long)blockIdx.x * HW;
-  const float4* xin = reinterpret_cast<const float4*>(x + tok0 * C);
-  for (int i = threadIdx.x; i < HW * C4; i += blockDim.x) xs4[i] = xin[i];
-  __syncthreads();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-  for (int t = warp; t < HW; t += nw) {
-    const int xx = t % W, yy = t / W;
-    const long long tok = tok0 + t;
-    float4 v[8];
-    float s = 0.f;
-    int n = 0;
-    for (int c = lane; c < C4; c += 32, ++n) {
-      float4 acc = reinterpret_cast<const float4*>(bias)[c];
-#pragma unroll
-      for (int ky = 0; ky < 3; ++ky) {
-        const int sy = yy + ky - 1;
-        if (sy < 0 || sy >= H) continue;
-#pragma unroll
-        for (int kx = 0; kx < 3; ++kx) {
-          const int sx = xx + kx - 1;
-          if (sx < 0 || sx >= W) continue;
-          const float4 xv = xs4[(t + (ky - 1) * W + (kx - 1)) * C4 + c];
-          const float4 wv = reinterpret_cast<const float4*>(w9c + (ky * 3 + kx) * C)[c];
-          acc.x += xv.x * wv.x; acc.y += xv.y * wv.y; acc.z += xv.z * wv.z; acc.w += xv.w * wv.w;
-        }
-      }
-      const float4 xc = xs4[t * C4 + c];
-      acc.x += xc.x; acc.y += xc.y; acc.z += xc.z; acc.w += xc.w;
-      reinterpret_cast<float4*>(y + tok * C)[c] = acc;
-      v[n] = acc;
-      s += (acc.x + acc.y) + (acc.z + acc.w);
-    }
-    const float mean = warp_sum(s) / float(C);
-    float q = 0.f;
-    for (int i = 0; i < n; ++i) {
-      const float dx = v[i].x - mean, dy = v[i].y - mean, dz = v[i].z - mean, dw = v[i].w - mean;
-      q += (dx * dx + dy * dy) + (dz * dz + dw * dw);
-    }
-    const float rstd = rsqrtf(warp_sum(q) / float(C) + eps);
-    n = 0;
-    __half* orow = o16 + tok * (split ? 2 * C : C);
-    for (int c = lane; c < C4; c += 32, ++n) {
-      const float4 gg = reinterpret_cast<const float4*>(g)[c], bb = reinterpret_cast<const float4*>(bt)[c];
-      float4 o;
-      o.x = (v[n].x - mean) * rstd * gg.x + bb.x; o.y = (v[n].y - mean) * rstd * gg.y + bb.y;
-      o.z = (v[n].z - mean) * rstd * gg.z + bb.z; o.w = (v[n].w - mean) * rstd * gg.w + bb.w;
-      store_act4(orow, 4 * c, split, o);
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------- depthwise 3x3 + residual
-// y = dwconv3x3(x) + bias + x   (hf:models/florence2/modeling_florence2.py:281,293 and :431,443)
-__global__ void dwconv3x3_res_kernel(const float* __restrict__ x, int B, int H, int W, int C,
-                                     const float* __restrict__ w /*[9][C]*/, const float* __restrict__ bias,
-                                     float* __restrict__ y) {
-  pdl_wait();   // PDL: inputs come from the previous kernel in the stream
-  const long long n = (long long)B * H * W * C;
-  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-    const int c = int(i % C);
-    long long p = i / C;
-    const int xx = int(p % W); p /= W;
-    const int yy = int(p % H);
-    const int b = int(p / H);
-    float acc = bias[c];
-#pragma unroll
-    for (int ky = 0; ky < 3; ++ky) {
-      const int sy = yy + ky - 1;
-      if (sy < 0 || sy >= H) continue;
-#pragma unroll
-      for (int kx = 0; kx < 3; ++kx) {
-        const int sx = xx + kx - 1;
-        if (sx < 0 || sx >= W) continue;
-        acc += x[(((long long)b * H + sy) * W + sx) * C + c] * w[(ky * 3 + kx) * C + c];
-      }
-    }
-    y[i] = acc + x[i];
-  }
-}
-
 // ---------------------------------------------------------------------------------------- window attention
 // qkv fp16 [B*H*W][3C] for REAL tokens only.  The reference zero-pads the normed map to a multiple of the 12x12
 // window; padded tokens have qkv = bias and take part as keys/values unmasked
 // (hf:models/florence2/modeling_florence2.py:346-350,377-383).  Exact shortcut: one "pad key" (k = bias_k,
 // v = bias_v) with multiplicity n_pad = 144 - n_real.  One CTA per (batch, window, head); one thread per query.
-// QB queries per thread (t, t + ceil(nreal / QB), ...): every K / V row read from shared memory feeds QB independent
-// online-softmax chains.  Only QB = 1 is instantiated (see b2p_window_attn).
-template <int D, int QB>
-__global__ void window_attn_kernel(const float* __restrict__ qkv, const float* __restrict__ qkv_bias, int B, int H,
-                                   int W, int C, int heads, int win, __half* __restrict__ out, int split, int kv_cap) {
+__global__ void window_attn_kernel(const float* __restrict__ qkv, const float* __restrict__ qkv_bias, int B, int H, int W,
+                                   int C, int heads, int win, __half* __restrict__ out, int split, int kv_cap) {
   pdl_wait();   // PDL: inputs come from the previous kernel in the stream
   extern __shared__ float4 sm4[];
-  constexpr int D4 = D / 4;
+  constexpr int D = 32, D4 = D / 4;
   const int nwx = (W + win - 1) / win, nwy = (H + win - 1) / win;
   int bid = blockIdx.x;
   const int head = bid % heads; bid /= heads;
@@ -311,84 +154,58 @@ __global__ void window_attn_kernel(const float* __restrict__ qkv, const float* _
   }
   __syncthreads();
   const float scale = rsqrtf(float(D));
-  const int nq = (nreal + QB - 1) / QB;
-  for (int t0 = threadIdx.x; t0 < nq; t0 += blockDim.x) {
-    long long tok[QB];
-    bool live[QB];
-    float4 q[QB][D4], acc[QB][D4];
-    float m[QB], l[QB];
+  for (int t = threadIdx.x; t < nreal; t += blockDim.x) {
+    const long long tok = ((long long)b * H + y0 + t / nx) * W + x0 + t % nx;
+    float4 q[D4], acc[D4];
 #pragma unroll
-    for (int u = 0; u < QB; ++u) {
-      const int t = t0 + u * nq;
-      live[u] = t < nreal;
-      const int tc = live[u] ? t : t0;      // a dead slot recomputes query t0 and stores nothing
-      tok[u] = ((long long)b * H + y0 + tc / nx) * W + x0 + tc % nx;
+    for (int d = 0; d < D4; ++d) {
+      q[d] = reinterpret_cast<const float4*>(qkv + tok * 3 * C + head * D)[d];
+      q[d].x *= scale; q[d].y *= scale; q[d].z *= scale; q[d].w *= scale;
+      acc[d] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    float m = -INFINITY, l = 0.f;
+    if (npad > 0) {
+      float s = 0.f;
 #pragma unroll
       for (int d = 0; d < D4; ++d) {
-        q[u][d] = reinterpret_cast<const float4*>(qkv + tok[u] * 3 * C + head * D)[d];
-        q[u][d].x *= scale; q[u][d].y *= scale; q[u][d].z *= scale; q[u][d].w *= scale;
-        acc[u][d] = make_float4(0.f, 0.f, 0.f, 0.f);
+        const float4 kb = reinterpret_cast<const float4*>(qkv_bias + C + head * D)[d];
+        s += (q[d].x * kb.x + q[d].y * kb.y) + (q[d].z * kb.z + q[d].w * kb.w);
       }
-      m[u] = -INFINITY; l[u] = 0.f;
-    }
-    if (npad > 0) {
+      m = s;
+      l = float(npad);
 #pragma unroll
-      for (int u = 0; u < QB; ++u) {
-        float s = 0.f;
-#pragma unroll
-        for (int d = 0; d < D4; ++d) {
-          const float4 kb = reinterpret_cast<const float4*>(qkv_bias + C + head * D)[d];
-          s += (q[u][d].x * kb.x + q[u][d].y * kb.y) + (q[u][d].z * kb.z + q[u][d].w * kb.w);
-        }
-        m[u] = s;
-        l[u] = float(npad);
-#pragma unroll
-        for (int d = 0; d < D4; ++d) {
-          const float4 vb = reinterpret_cast<const float4*>(qkv_bias + 2 * C + head * D)[d];
-          acc[u][d] = make_float4(l[u] * vb.x, l[u] * vb.y, l[u] * vb.z, l[u] * vb.w);
-        }
+      for (int d = 0; d < D4; ++d) {
+        const float4 vb = reinterpret_cast<const float4*>(qkv_bias + 2 * C + head * D)[d];
+        acc[d] = make_float4(l * vb.x, l * vb.y, l * vb.z, l * vb.w);
       }
     }
     for (int j = 0; j < nreal; ++j) {
-      float s[QB], p[QB];
-#pragma unroll
-      for (int u = 0; u < QB; ++u) s[u] = 0.f;
+      float s = 0.f;
 #pragma unroll
       for (int d = 0; d < D4; ++d) {
         const float4 kk = Ks[j * D4 + d];
-#pragma unroll
-        for (int u = 0; u < QB; ++u) s[u] += (q[u][d].x * kk.x + q[u][d].y * kk.y) + (q[u][d].z * kk.z + q[u][d].w * kk.w);
+        s += (q[d].x * kk.x + q[d].y * kk.y) + (q[d].z * kk.z + q[d].w * kk.w);
       }
+      if (s > m) {
+        const float r = __expf(m - s);
+        l *= r;
 #pragma unroll
-      for (int u = 0; u < QB; ++u) {
-        if (s[u] > m[u]) {
-          const float r = __expf(m[u] - s[u]);
-          l[u] *= r;
-#pragma unroll
-          for (int d = 0; d < D4; ++d) { acc[u][d].x *= r; acc[u][d].y *= r; acc[u][d].z *= r; acc[u][d].w *= r; }
-          m[u] = s[u];
-        }
-        p[u] = __expf(s[u] - m[u]);
-        l[u] += p[u];
+        for (int d = 0; d < D4; ++d) { acc[d].x *= r; acc[d].y *= r; acc[d].z *= r; acc[d].w *= r; }
+        m = s;
       }
+      const float p = __expf(s - m);
+      l += p;
 #pragma unroll
       for (int d = 0; d < D4; ++d) {
         const float4 vv = Vs[j * D4 + d];
-#pragma unroll
-        for (int u = 0; u < QB; ++u) {
-          acc[u][d].x += p[u] * vv.x; acc[u][d].y += p[u] * vv.y; acc[u][d].z += p[u] * vv.z; acc[u][d].w += p[u] * vv.w;
-        }
+        acc[d].x += p * vv.x; acc[d].y += p * vv.y; acc[d].z += p * vv.z; acc[d].w += p * vv.w;
       }
     }
+    const float inv = 1.f / l;
+    __half* orow = out + tok * (split ? 2 * C : C);
 #pragma unroll
-    for (int u = 0; u < QB; ++u) {
-      if (!live[u]) continue;
-      const float inv = 1.f / l[u];
-      __half* orow = out + tok[u] * (split ? 2 * C : C);
-#pragma unroll
-      for (int d = 0; d < D4; ++d)
-        store_act4(orow, head * D + 4 * d, split, make_float4(acc[u][d].x * inv, acc[u][d].y * inv, acc[u][d].z * inv, acc[u][d].w * inv));
-    }
+    for (int d = 0; d < D4; ++d)
+      store_act4(orow, head * D + 4 * d, split, make_float4(acc[d].x * inv, acc[d].y * inv, acc[d].z * inv, acc[d].w * inv));
   }
 }
 
@@ -437,49 +254,6 @@ __global__ void __launch_bounds__(256) channel_attn_kernel(const float* __restri
   for (int n = w; n < N; n += 8) {
     const float* vr = base + (long long)n * 3 * C + 2 * C + g * D;
     const float vj = vr[j];
-    float acc = 0.f;
-#pragma unroll
-    for (int jj = 0; jj < D; ++jj) acc += pr[jj] * __shfl_sync(0xffffffffu, vj, jj);
-    store_act(out + ((long long)b * N + n) * (split ? 2 * C : C), g * D + j, split, acc);
-  }
-}
-
-// Small-N variant (split bit 1; the default since it was validated on the B200 in round 2, B2P_NO_CHATTN_SMALL=1 disables it): for
-// the 4x4 / 2x2 maps of the 64x64-crop mode (N <= 16 tokens) the 256-thread CTA above is almost all synchronisation; here
-// ONE WARP owns a (batch, group) pair, 4 pairs per CTA.  Same sums in the same order => bit-identical outputs.
-__global__ void __launch_bounds__(128) channel_attn_small_kernel(const float* __restrict__ qkv, int B, int N, int C, int groups,
-                                                                 __half* __restrict__ out, int split) {
-  pdl_wait();
-  constexpr int D = 32, NMAX = 16;
-  __shared__ float sm[4][2 * NMAX + D][D + 1];   // per warp: q rows [0,N), k rows [NMAX, NMAX+N), P rows [2*NMAX, 2*NMAX+32)
-  const int w = threadIdx.x >> 5, j = threadIdx.x & 31;
-  const int pair = blockIdx.x * 4 + w;
-  if (pair >= B * groups) return;
-  const int g = pair % groups, b = pair / groups;
-  float (*qs)[D + 1] = sm[w];
-  float (*ks)[D + 1] = sm[w] + NMAX;
-  float (*P)[D + 1] = sm[w] + 2 * NMAX;
-  const float* base = qkv + (long long)b * N * 3 * C;
-  for (int n = 0; n < N; ++n) {
-    qs[n][j] = base[(long long)n * 3 * C + g * D + j];
-    ks[n][j] = base[(long long)n * 3 * C + C + g * D + j];
-  }
-  __syncwarp();
-  const float sc = rsqrtf(float(N));
-  for (int i = 0; i < D; ++i) {
-    float s = 0.f;
-    for (int n = 0; n < N; ++n) s += qs[n][i] * ks[n][j];
-    const float v = s * sc;
-    const float m = warp_max(v);
-    const float e = __expf(v - m);
-    P[i][j] = e / warp_sum(e);
-  }
-  __syncwarp();
-  float pr[D];
-#pragma unroll
-  for (int jj = 0; jj < D; ++jj) pr[jj] = P[j][jj];
-  for (int n = 0; n < N; ++n) {
-    const float vj = base[(long long)n * 3 * C + 2 * C + g * D + j];
     float acc = 0.f;
 #pragma unroll
     for (int jj = 0; jj < D; ++jj) acc += pr[jj] * __shfl_sync(0xffffffffu, vj, jj);
@@ -776,28 +550,6 @@ int b2p_layernorm(const float* x, long long ldx, const float* gamma, const float
   return 0;
 }
 
-// out = LayerNorm(A * B^T + bias + residual): a park-only GEMM (raw partial accumulators of every (tile, k slice) in the
-// split-K workspace) followed by splitk_ln_kernel.  A, B as b2p_gemm (flags & 8: fp16x3 operands); residual fp32 [M][ldr];
-// out16: fp16 (flags & 4: [hi | lo], ld16 >= 2N) and / or out32: fp32.  Replaces b2p_gemm(+residual) + b2p_layernorm.
-int b2p_gemm_ln(const void* A, long long lda, const void* B, int M, int N, int K, const float* bias, const float* residual,
-                long long ldr, const float* gamma, const float* beta, float eps, void* out16, long long ld16, float* out32,
-                long long ld32, int flags, cudaStream_t st) {
-  if (M <= 0) return 0;
-  if (N % 16 || N > 1024 || (ldr % 4) || (ld32 % 4) || (ld16 % 4)) return set_error("gemm_ln: N must be a multiple of 16 and <= 1024, ld multiples of 4");
-  ParkInfo pk{};
-  ConvGemm d{};
-  d.mode = 0; d.bf16 = 0; d.A = A; d.lda = lda; d.B = B; d.M = M; d.N = N; d.K = K;
-  d.out = nullptr; d.ldc = N; d.out_f32 = 1; d.bias = nullptr; d.res = nullptr; d.ldr = 0; d.act = 0;
-  d.bn_max = (flags >> 8) & 0x1ff; d.x3 = (flags >> 3) & 1;
-  d.park = 1; d.park_info = &pk;
-  if (int e = gemm_launch(d, st)) return e;
-  const int wpb = 8;
-  launch_pdl(splitk_ln_kernel, dim3((M + wpb - 1) / wpb), dim3(wpb * 32), 0, st, pk, M, N, bias, residual, ldr, gamma, beta, eps,
-             (__half*)out16, ld16, out32, ld32, (flags & 4) ? N : 0);
-  B2P_CHECK_LAUNCH();
-  return 0;
-}
-
 int b2p_dwconv_ln(const float* x, int B, int H, int W, int C, const float* w9c, const float* bias, float* y,
                   const float* gamma, const float* beta, float eps, void* out16, int split, cudaStream_t st) {
   if (C % 4 || C > 1024) return set_error("dwconv_ln: C must be a multiple of 4 and <= 1024");
@@ -806,29 +558,8 @@ int b2p_dwconv_ln(const float* x, int B, int H, int W, int C, const float* w9c, 
     const int r = dwconv_ln_v3_launch(x, B, H, W, C, w9c, bias, y, gamma, beta, eps, out16, split & 1, st);
     if (r <= 0) return r;
   }
-  const size_t tile_bytes = size_t(H) * W * C * sizeof(float);
-  if ((split & 2) && tile_bytes <= 200 * 1024 && B > 0) {   // opt-in tiled variant (see dwconv_ln_tile_kernel)
-    static std::atomic<bool> attr{false};
-    if (!attr) {
-      if (cudaFuncSetAttribute(dwconv_ln_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess)
-        return set_error("dwconv_ln: cudaFuncSetAttribute failed");
-      attr = true;
-    }
-    const int threads = (H * W >= 16) ? 512 : 256;
-    launch_pdl(dwconv_ln_tile_kernel, dim3(B), dim3(threads), tile_bytes, st, x, H, W, C, w9c, bias, y, gamma, beta, eps, (__half*)out16,
-               (split & 1) ? C : 0);
-    B2P_CHECK_LAUNCH();
-    return 0;
-  }
   const int wpb = 8;
   launch_pdl(dwconv_ln_kernel, dim3(int((T + wpb - 1) / wpb)), dim3(wpb * 32), 0, st, x, B, H, W, C, w9c, bias, y, gamma, beta, eps, (__half*)out16, (split & 1) ? C : 0);
-  B2P_CHECK_LAUNCH();
-  return 0;
-}
-
-int b2p_dwconv3x3_res(const float* x, int B, int H, int W, int C, const float* w9c, const float* bias, float* y,
-                      cudaStream_t st) {
-  launch_pdl(dwconv3x3_res_kernel, dim3(grid_for((long long)B * H * W * C, 256)), dim3(256), 0, st, x, B, H, W, C, w9c, bias, y);
   B2P_CHECK_LAUNCH();
   return 0;
 }
@@ -849,16 +580,15 @@ int b2p_window_attn(const float* qkv, const float* qkv_bias, int B, int H, int W
   if (int e = bind_device()) return e;
   static std::atomic<bool> attr{false};
   if (!attr) {
-    cudaFuncSetAttribute(window_attn_kernel<32, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+    cudaFuncSetAttribute(window_attn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
     attr = true;
   }
   if (smem > 64 * 1024) return set_error("window_attn: window too large");
-  // (two queries per thread, QB = 2, measured SLOWER on the 16x16 map: 479 us against 357 -- 168 registers leave 12 warps per SM;
-  //  the one-window maps do use QB = 2, in window_attn_crop_kernel)
+  // (two queries per thread measured slower on the 16x16 map, 479 us against 357: 168 registers leave 12 warps per SM)
   // one thread per query of the window: small maps (4x4, 8x8 in the 64x64-crop mode) get small CTAs so more of them fit per SM
   const int nq = kv_cap;
   const int threads = nq >= 160 ? 160 : ((nq + 31) / 32) * 32;
-  launch_pdl(window_attn_kernel<32, 1>, dim3(B * nw * heads), dim3(threads), smem, st, qkv, qkv_bias, B, H, W, C, heads, win, (__half*)out, (split & 1) ? C : 0, kv_cap);
+  launch_pdl(window_attn_kernel, dim3(B * nw * heads), dim3(threads), smem, st, qkv, qkv_bias, B, H, W, C, heads, win, (__half*)out, (split & 1) ? C : 0, kv_cap);
   B2P_CHECK_LAUNCH();
   return 0;
 }
@@ -868,11 +598,6 @@ int b2p_channel_attn(const float* qkv, int B, int N, int C, int groups, void* ou
   if (split & 4) {   // register-tiled kernel, florence_simt.cu
     const int r = channel_attn_v3_launch(qkv, B, N, C, groups, out, split & 1, st);
     if (r <= 0) return r;
-  }
-  if ((split & 2) && N <= 16 && B > 0) {   // opt-in small-N variant (see channel_attn_small_kernel)
-    launch_pdl(channel_attn_small_kernel, dim3((B * groups + 3) / 4), dim3(128), 0, st, qkv, B, N, C, groups, (__half*)out, (split & 1) ? C : 0);
-    B2P_CHECK_LAUNCH();
-    return 0;
   }
   launch_pdl(channel_attn_kernel, dim3(B * groups), dim3(256), 0, st, qkv, N, C, groups, (__half*)out, (split & 1) ? C : 0);
   B2P_CHECK_LAUNCH();

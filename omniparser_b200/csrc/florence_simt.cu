@@ -3,8 +3,9 @@
 // token re-read its nine depthwise taps and weights through L1, every (crop, head) was a one-warp CTA, the channel attention
 // ran its softmax as 64 butterfly reductions per group.  Here a CTA owns a tile that fits shared memory, loads it once with
 // coalesced 16-byte accesses, keeps per-thread constants (depthwise weights, probability rows) in registers, and writes
-// whole rows back.  Selected by split bit 2 (value 4) of the C-ABI entry points; the first versions stay as the checkers
-// (tests/test_ops_gpu.py compares both) and for shapes these do not cover (768-mode maps).
+// whole rows back.  Selected by split bit 2 (value 4) of the C-ABI entry points; without it, and for shapes these do not
+// cover (768-mode maps), the entry points run the first versions, which also serve as the checkers (tests/test_ops_gpu.py
+// compares both).
 // Reference math: hf:models/florence2/modeling_florence2.py (ConvPosEnc 281-293, WindowAttention 346-383,
 // ChannelAttention 228-264), hf:models/bart/modeling_bart.py:143-258.
 #include "ptx.cuh"
@@ -566,17 +567,15 @@ int channel_attn_v3_launch(const float* qkv, int B, int N, int C, int groups, vo
 // warp re-reads the head's K and V rows (430 MB of L2 -> SM traffic per launch).  Here one warp owns a (batch, head): K and V
 // (<= 16 keys, 2 values per lane per key) stay in registers and the queries are processed in turn with exactly the
 // arithmetic of mha_kernel (four keys per step, then the tail) => bit-identical outputs.
-constexpr int kMhaLmax = 16, kMhaQSplit = 1;   // > 1 deals the queries of a head to several warps: measured slower (4: 48 us vs 38)
+// (dealing the queries of one head to several warps measured slower: 4 warps, 48 us against 38)
+constexpr int kMhaLmax = 16;
 __global__ void __launch_bounds__(128) mha_short_kernel(const float* __restrict__ qp, long long ldq, const float* __restrict__ kp,
                                                         const float* __restrict__ vp, long long ldk, int B, int Lq, int Lk, int heads,
                                                         __half* __restrict__ out, long long ldo, int split) {
   pdl_wait();
-  const int wid0 = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int wid = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
-  if (wid0 >= B * heads * kMhaQSplit) return;
-  // the queries of one (batch, head) are dealt to kMhaQSplit warps (each query is a long dependent chain of butterfly
-  // reductions: one warp per head left the SM latency-bound at 38 us per launch); K / V re-loads hit L1 / L2
-  const int part = wid0 % kMhaQSplit, wid = wid0 / kMhaQSplit;
+  if (wid >= B * heads) return;
   const int h = wid % heads, b = wid / heads;
   const float* kb = kp + (long long)b * Lk * ldk + h * 64;
   const float* vb = vp + (long long)b * Lk * ldk + h * 64;
@@ -594,12 +593,11 @@ __global__ void __launch_bounds__(128) mha_short_kernel(const float* __restrict_
   // the query loop stays ROLLED (fully unrolled it is ~11k instructions and thrashes the instruction cache: 112 us per launch
   // against 40); the next query's row is fetched one iteration ahead so its L2 round trip overlaps this query's arithmetic
   const float* qrow = qp + (long long)b * Lq * ldq + h * 64 + 2 * lane;
-  if (part >= Lq) return;
-  float2 qn = *reinterpret_cast<const float2*>(qrow + (long long)part * ldq);
+  float2 qn = *reinterpret_cast<const float2*>(qrow);
 #pragma unroll 1
-  for (int qi = part; qi < Lq; qi += kMhaQSplit) {
+  for (int qi = 0; qi < Lq; ++qi) {
     float2 q = qn;
-    if (qi + kMhaQSplit < Lq) qn = *reinterpret_cast<const float2*>(qrow + (long long)(qi + kMhaQSplit) * ldq);
+    if (qi + 1 < Lq) qn = *reinterpret_cast<const float2*>(qrow + (long long)(qi + 1) * ldq);
     q.x *= 0.125f; q.y *= 0.125f;
     float m = -INFINITY, l = 0.f;
     float2 acc = make_float2(0.f, 0.f);
@@ -654,7 +652,7 @@ __global__ void __launch_bounds__(128) mha_short_kernel(const float* __restrict_
 int mha_short_launch(const float* q, long long ldq, const float* k, const float* v, long long ldk, int B, int Lq, int Lk, int heads,
                      void* out, long long ldo, int split, cudaStream_t st) {
   if (Lk > kMhaLmax || Lq > kMhaLmax || Lq < 2 || B <= 0) return 1;
-  const int total = B * heads * kMhaQSplit;
+  const int total = B * heads;
   launch_pdl(mha_short_kernel, dim3((total + 3) / 4), dim3(128), 0, st, q, ldq, k, v, ldk, B, Lq, Lk, heads, (__half*)out, ldo,
              split ? heads * 64 : 0);
   cudaError_t e = cudaGetLastError();

@@ -86,8 +86,6 @@ struct GemmArgs {
   float* ws;   // split-K partial tiles [tile][slice][128][bn] fp32
   int* counters;   // split-K {arrived, finished} counters per output tile (self-resetting)
   int sk_last;     // split-K variant: 1 = last arriver reduces (wait-free, B2P_SPLITK_LAST=1), 0 = distributed reduction
-  int park;        // 1 = park-only: every (tile, k slice) leaves its raw fp32 accumulators in ws and the kernel ends; the
-                   // following kernel (splitk_ln_kernel) sums the slices, adds bias + residual and applies LayerNorm
   unsigned long long* trace;   // B2P_TRACE build of the kernel only: [CTA][16] globaltimer stamps (see trace_stamp)
 };
 
@@ -638,7 +636,7 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
       tc_fence_after();
       if constexpr (kTrace) { if (item == blockIdx.x && threadIdx.x == 64) trace_stamp<kTrace>(g, kTrFirstEpiStart); }
       const uint32_t t_row = tmem_base + (uint32_t(grp * 32) << 16) + uint32_t(acc * 256);
-      if (e_ksplit == 1 && !g.park) {
+      if (e_ksplit == 1) {
         // the accumulator goes back to the MMA warp as soon as this warp's LAST 16-column chunk sits in registers (before it
         // is processed).  (A software-pipelined variant with two register buffers measured no faster and spilled.)
         bool released = false;
@@ -665,7 +663,7 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
           if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);
         }
       } else {
-        // split-K: every slice parks its raw fp32 partial tile, then the partials are summed in slice order (deterministic) and
+        // split-K: every slice stores its raw fp32 partial tile, then the partials are summed in slice order (deterministic) and
         // the epilogue runs -- by the last CTA to arrive (sk_last: nobody waits for anybody, so partially resident grids cannot
         // deadlock) or, by default, distributed over the tile's ksplit CTAs (faster, see below).
         float* wsp = g.ws + ((size_t(tile) * e_ksplit + ks) * kTileM + r) * e_bn;
@@ -681,9 +679,7 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);
-        if (g.park) {
-          // park-only: nothing to wait for, nothing to reduce here (the consumer kernel starts after this grid has completed)
-        } else if (g.sk_last) {
+        if (g.sk_last) {
           __threadfence();
           asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
           volatile uint32_t* s_last = tmem_slot + 1;
@@ -938,7 +934,7 @@ static int device_setup() {
 // Choose the N tile and the split-K factor with a small time model (microseconds per CTA):
 //   per k-block  max(MMA issue, smem fill): MMA = bn*bk/32 cycles at ~1.9 GHz; fill = (A + B bytes) / ~70 GB/s per SM
 //   (measured: L2 -> SM delivery tops out near 12 TB/s chip-wide, profiles/r1_gemm_notes.md)
-//   per item     ~2.5 us pipeline fill/drain + epilogue (~0.012 us per output column) + split-K park/reduce.
+//   per item     ~2.5 us pipeline fill/drain + epilogue (~0.012 us per output column) + split-K partial store/reduce.
 static void pick_tiling(int N, int m_tiles, int num_kb, int bk, uint32_t a_bytes, int bn_max, bool allow_split, bool x3,
                         int* bn_out, int* ksplit_out) {
   static const int cand[] = {256, 192, 128, 96, 64, 48, 32, 16};
@@ -979,12 +975,12 @@ static void pick_tiling(int N, int m_tiles, int num_kb, int bk, uint32_t a_bytes
       if (ks > 1 && size_t(tiles) * ks * 128 * c * 4 > kWsBytes) continue;
       const long items = tiles * ks;
       const long waves = (items + g_num_sms - 1) / g_num_sms;
-      // split-K overhead: park one fp32 partial tile + read one tile's worth back (distributed reduce) at ~100 GB/s/SM
+      // split-K overhead: store one fp32 partial tile + read one tile's worth back (distributed reduce) at ~100 GB/s/SM
       double t_split = ks > 1 ? 2.0 + 2.0 * (128.0 * c * 4.0 / 100000.0) : 0.0;
       double t_kb_ = t_kb;
       double occupancy_penalty = 0.0;
       if (few_ctas && waves == 1) {
-        // measured (profiles/r2_notes.md 2): a single-wave launch takes ~11 us whatever its tiling (split-K's park / arrive /
+        // measured (profiles/r2_notes.md 2): a single-wave launch takes ~11 us whatever its tiling (split-K's store / arrive /
         // reduce costs ~6 us, a CTA of a sparse grid fills at ~100 GB/s), so equal-latency tilings are resolved by a charge per
         // occupied SM: the sparser grid leaves SMs to the other streams of the pipelined parser (bench: 19.2 -> 18.1 ms/step)
         if (ks > 1) t_split = 5.0 + double(ks) * (128.0 * c * 4.0 / 100000.0);
@@ -1137,12 +1133,6 @@ int gemm_launch(const ConvGemm& d, cudaStream_t st) {
       if (res_stagesA > 8) res_stagesA = 8;
     }
   }
-  if (d.park) {
-    if (d.mode != 0 || slot < 0) return set_error("gemm (park-only): needs mode 0 and a split-K workspace slot for this stream");
-    if (size_t(g.m_tiles) * ((d.N + bn - 1) / bn) * ksplit * 128 * bn * 4 > kWsBytes) return set_error("gemm (park-only): partial tiles exceed the workspace");
-    bres = false;
-  }
-  g.park = d.park ? 1 : 0;
   g.bres = bres ? 1 : 0;
   g.sep = (halo || bres) ? 1 : 0;
   g.taps = halo ? 9 : 1;
@@ -1241,10 +1231,6 @@ int gemm_launch(const ConvGemm& d, cudaStream_t st) {
   if (ce == cudaSuccess) ce = cudaGetLastError();
   if (ce != cudaSuccess) return set_error(cudaGetErrorString(ce));
   count_launch();
-  if (d.park_info) {
-    d.park_info->ws = g.ws; d.park_info->bn = bn; d.park_info->ksplit = g.ksplit; d.park_info->n_tiles = g.n_tiles;
-    d.park_info->m_tiles = g.m_tiles; d.park_info->mt_fast = g.mt_fast;
-  }
   return 0;
 }
 

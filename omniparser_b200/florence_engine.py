@@ -178,17 +178,6 @@ class FlorencePlan:
         assert size in (64, 768)
         self.S = size
         self.tag = f"florence{instance}"
-        # smem-tiled dwconv+LN and warp-per-group channel attention (N <= 16): bit-identical with the per-token / per-CTA kernels
-        # (tests/test_ops_gpu.py, validated on the B200 in round 2); B2P_NO_DWCONV_TILE / B2P_NO_CHATTN_SMALL select the old ones
-        self.dw_tile = not os.environ.get("B2P_NO_DWCONV_TILE")
-        self.ca_small = not os.environ.get("B2P_NO_CHATTN_SMALL")
-        # round-2 SIMT kernels (csrc/florence_simt.cu): strip dwconv+LN, per-image window attention, register-tiled channel
-        # attention, warp-per-head short attention; B2P_NO_SIMT_V3=1 selects the first versions (the checkers)
-        self.v3 = not os.environ.get("B2P_NO_SIMT_V3")
-        # B2P_GEMM_LN=1: decoder out-proj / cross out-proj / fc2 as park-only split-K GEMM + one reduce/LayerNorm kernel
-        # (b2p_gemm_ln) instead of GEMM with in-kernel split-K reduction + LayerNorm launch.  Bit-identical; measured neutral
-        # on B200 (decode step 0.84 vs 0.82 ms: the kernel boundary costs what the in-kernel wait cost), so it stays opt-in.
-        self.fuse_ln = bool(os.environ.get("B2P_GEMM_LN"))
         self.warmed = False
         import threading
         self.lock = threading.Lock()
@@ -219,7 +208,6 @@ class FlorencePlan:
         self._build_decoder()
         self.g_enc = None
         self.g_enc_nr = None
-        self._forked = False
 
     # ------------------------------------------------------------------ helpers
     def _e(self, *shape, dt=torch.float32):
@@ -252,21 +240,6 @@ class FlorencePlan:
         lst.append(lambda: ops.gemm(a, a.stride(0), lin.w, M, lin.N, lin.K, out, out.stride(0), lin.b, res,
                                     res.stride(0) if res is not None else 0, act, out_f32=(out.dtype == torch.float32),
                                     split=split, x3=self.x3))
-
-    def _gemm_ln(self, lst, a, lin, res, ln, o16, o32, enc=False):
-        """o16 / o32 = LayerNorm(a @ W^T + b + res): one park-only GEMM + the split-K-reduce / LayerNorm kernel (b2p_gemm_ln)
-        instead of GEMM (+ in-kernel split-K reduction) + LayerNorm.  Same sums in the same order."""
-        M = a.shape[0]
-        assert a.shape[1] == self.KX * lin.K and res.dtype == torch.float32
-        f = 2 * M * lin.N * lin.Klog
-        if enc:
-            self.flops_enc += f
-        else:
-            self.flops_dec += f
-        f_ = lambda: ops.gemm_ln(a, a.stride(0), lin.w, M, lin.N, lin.K, lin.b, res, res.stride(0), ln.g, ln.b,
-                                 o16, o16.stride(0), o32, o32.stride(0), split=self.x3, x3=self.x3)
-        f_.n_kernels = 2        # launch accounting of graph replays (ops.count_graph_launches)
-        lst.append(f_)
 
     def _ln(self, lst, x, ln, T, C, o16=None, o32=None):
         lst.append(lambda: ops.layernorm(x, ln.g, ln.b, T, C, o16, o32, split=self.x3))
@@ -325,20 +298,20 @@ class FlorencePlan:
                     act_, qkv, f = self._pool("act", T, C, act=True), self._pool("qkv", T, 3 * C), self._pool("f", T, 4 * C, act=True)
                     x1, h = xA, act_
                     ops_.append(lambda x=x, x1=x1, h=h, e=e, H=H, C=C: ops.dwconv_ln(x, K, H, H, C, e["dw1_w"], e["dw1_b"], x1,
-                                                                                 e["n1"].g, e["n1"].b, h, split=x3, tile=self.dw_tile, v3=self.v3))
+                                                                                 e["n1"].g, e["n1"].b, h, split=x3, v3=True))
                     self._gemm(ops_, h, e["qkv"], qkv)
                     a = act_
                     if kind == "spatial_block":
                         hd = w.heads[s]
-                        ops_.append(lambda qkv=qkv, a=a, e=e, H=H, C=C, hd=hd: ops.window_attn(qkv, e["qkv"].b, K, H, H, C, hd, a, split=x3, v3=self.v3))
+                        ops_.append(lambda qkv=qkv, a=a, e=e, H=H, C=C, hd=hd: ops.window_attn(qkv, e["qkv"].b, K, H, H, C, hd, a, split=x3, v3=True))
                     else:
                         gr = w.groups[s]
-                        ops_.append(lambda qkv=qkv, a=a, H=H, C=C, gr=gr: ops.channel_attn(qkv, K, H * H, C, gr, a, split=x3, small=self.ca_small, v3=self.v3))
+                        ops_.append(lambda qkv=qkv, a=a, H=H, C=C, gr=gr: ops.channel_attn(qkv, K, H * H, C, gr, a, split=x3, v3=True))
                     x2 = xB
                     self._gemm(ops_, a, e["proj"], x2, res=x1)
                     x3_, h2 = xA, act_
                     ops_.append(lambda x2=x2, x3_=x3_, h2=h2, e=e, H=H, C=C: ops.dwconv_ln(x2, K, H, H, C, e["dw2_w"], e["dw2_b"], x3_,
-                                                                                      e["n2"].g, e["n2"].b, h2, split=x3, tile=self.dw_tile, v3=self.v3))
+                                                                                      e["n2"].g, e["n2"].b, h2, split=x3, v3=True))
                     self._gemm(ops_, h2, e["fc1"], f, act=ACT_GELU, split=x3)
                     x4 = xB
                     self._gemm(ops_, f, e["fc2"], x4, res=x3_)
@@ -368,7 +341,7 @@ class FlorencePlan:
             qkv, f = self._pool("eqkv", TE, 3 * D), self._pool("ef", TE, 4 * D, act=True)
             self._gemm(ops_, h, lay["qkv"], qkv)
             a = h if self.pool else self._act(TE, D)
-            ops_.append(lambda qkv=qkv, a=a: ops.mha(qkv, 3 * D, qkv[:, D:], qkv[:, 2 * D:], 3 * D, K, L, L, self.HEADS, a, a.stride(0), split=x3, v3=self.v3))
+            ops_.append(lambda qkv=qkv, a=a: ops.mha(qkv, 3 * D, qkv[:, D:], qkv[:, 2 * D:], 3 * D, K, L, L, self.HEADS, a, a.stride(0), split=x3, v3=True))
             y = self._pool("ey", TE, D)
             self._gemm(ops_, a, lay["o"], y, res=x)
             if not self.pool:
@@ -390,31 +363,15 @@ class FlorencePlan:
 
     # ------------------------------------------------------------------ one greedy decode step
     def _build_decoder(self):
-        """The decode step is ~70 small, latency-bound launches.  The crop rows CAN be split into `parts` independent
-        chains (own KV cache, step counter, CUDA graph, stream) replayed concurrently; on B200 that measured slower
-        (every chain re-streams the 0.5 GB of decoder weights), so the default is one chain."""
-        K = self.K
-        P = int(os.environ.get("B2P_DECODE_PARTS", "1"))   # measured: 2 chains -8 %, 3 chains -16 % (weights stream twice)
-        if K < 64 * P:
-            P = 1
-        per = (K // P + 15) // 16 * 16 if P > 1 else K
-        self.parts = []
-        r0 = 0
-        for i in range(P):
-            r1 = K if i == P - 1 else min(K, r0 + per)
-            self.parts.append(self._build_dec_part(i, r0, r1))
-            r0 = r1
-        self.dec_ops = [f for pt in self.parts for f in pt["ops"]]   # (counting / introspection only)
-
-    def _build_dec_part(self, idx, r0, r1):
-        w, D, x3 = self.w, self.D, self.x3
-        R = r1 - r0
+        """The decode step: ~70 small, latency-bound launches over all K crop rows.  (Splitting the rows into concurrent
+        chains measured slower on B200, -8 % with 2 chains: every chain re-streams the 0.5 GB of decoder weights.)"""
+        w, D, x3, R = self.w, self.D, self.x3, self.K
         g = w.gen
         tmax = self.max_len
-        ops_ = []
-        seq, finished, logits = self.seq[r0:r1], self.finished[r0:r1], self.logits[r0:r1]
-        step = torch.zeros((1,), dtype=torch.int32, device=self.dev)
-        n_unf = torch.zeros((1,), dtype=torch.int32, device=self.dev)
+        ops_ = self.dec_ops
+        seq, finished, logits = self.seq, self.finished, self.logits
+        self.step = step = torch.zeros((1,), dtype=torch.int32, device=self.dev)
+        self.n_unf = n_unf = torch.zeros((1,), dtype=torch.int32, device=self.dev)
         e0 = self._e(R, D)
         ops_.append(lambda: ops.decoder_embed(w.E32, seq, seq.stride(0), step, w.dec_pos, R, D, e0))
         x = self._e(R, D); h = self._act(R, D)
@@ -427,64 +384,51 @@ class FlorencePlan:
             a = self._act(R, D)
             ops_.append(lambda qkv=qkv, kc=kc, vc=vc, a=a: ops.mha_cached(qkv, 3 * D, qkv[:, D:], qkv[:, 2 * D:], 3 * D, kc, vc, tmax,
                                                                        step, R, self.HEADS, a, a.stride(0), split=x3))
-            if self.fuse_ln:
-                xn = self._e(R, D); h = self._act(R, D)
-                self._gemm_ln(ops_, a, lay["o"], x, lay["ln1"], h, xn)
-                x = xn
-            else:
-                y = self._e(R, D)
-                self._gemm(ops_, a, lay["o"], y, res=x, enc=False)
-                x = self._e(R, D); h = self._act(R, D)
-                self._ln(ops_, y, lay["ln1"], R, D, h, x)
+            y = self._e(R, D)
+            self._gemm(ops_, a, lay["o"], y, res=x, enc=False)
+            x = self._e(R, D); h = self._act(R, D)
+            self._ln(ops_, y, lay["ln1"], R, D, h, x)
             q = self._e(R, D)
             self._gemm(ops_, h, lay["cq"], q, enc=False)
-            kv = self.cross_kv[li][r0 * self.L:r1 * self.L]
+            kv = self.cross_kv[li]
             a2 = self._act(R, D)
             ops_.append(lambda q=q, kv=kv, a2=a2: ops.mha(q, D, kv, kv[:, D:], 2 * D, R, 1, self.L, self.HEADS, a2, a2.stride(0), split=x3))
-            if self.fuse_ln:
-                xn = self._e(R, D); h = self._act(R, D)
-                self._gemm_ln(ops_, a2, lay["co"], x, lay["ln2"], h, xn)
-                x = xn
-            else:
-                y = self._e(R, D)
-                self._gemm(ops_, a2, lay["co"], y, res=x, enc=False)
-                x = self._e(R, D); h = self._act(R, D)
-                self._ln(ops_, y, lay["ln2"], R, D, h, x)
+            y = self._e(R, D)
+            self._gemm(ops_, a2, lay["co"], y, res=x, enc=False)
+            x = self._e(R, D); h = self._act(R, D)
+            self._ln(ops_, y, lay["ln2"], R, D, h, x)
             f = self._act(R, 4 * D)
             self._gemm(ops_, h, lay["fc1"], f, act=ACT_GELU, enc=False, split=x3)
-            if self.fuse_ln:
-                xn = self._e(R, D); h = self._act(R, D)
-                self._gemm_ln(ops_, f, lay["fc2"], x, lay["ln3"], h, xn)
-                x = xn
-            else:
-                y = self._e(R, D)
-                self._gemm(ops_, f, lay["fc2"], y, res=x, enc=False)
-                x = self._e(R, D); h = self._act(R, D)
-                self._ln(ops_, y, lay["ln3"], R, D, h, x)
+            y = self._e(R, D)
+            self._gemm(ops_, f, lay["fc2"], y, res=x, enc=False)
+            x = self._e(R, D); h = self._act(R, D)
+            self._ln(ops_, y, lay["ln3"], R, D, h, x)
         lm = type("W", (), {})()
         lm.w, lm.b, lm.N, lm.K, lm.Klog = w.E16, None, w.vocab, D, D
         self._gemm(ops_, h, lm, logits, enc=False)
         fb = g.get("forced_bos_token_id")
         fe = g.get("forced_eos_token_id")
-        pick = lambda dump=None: ops.greedy_pick(logits, logits.stride(0), w.vocab, R, seq, seq.stride(0), finished, step,
-                                                 g.get("no_repeat_ngram_size", 0) or 0, -1 if fb is None else fb,
-                                                 -1 if fe is None else fe, g["eos_token_id"], g["pad_token_id"], self.max_len,
-                                                 dump, n_unf)
+        self.pick = lambda dump=None: ops.greedy_pick(logits, logits.stride(0), w.vocab, R, seq, seq.stride(0), finished, step,
+                                                      g.get("no_repeat_ngram_size", 0) or 0, -1 if fb is None else fb,
+                                                      -1 if fe is None else fe, g["eos_token_id"], g["pad_token_id"], self.max_len,
+                                                      dump, n_unf)
+        tail = [lambda: self.pick(None), lambda: ops.step_advance(step)]
+        self.dec_full = ops_ + tail
         # Steps whose token is forced by the generation config (forced BOS at length 1, forced EOS at the last length:
         # hf:generation/logits_process.py:1552,1597) never look at the logits: the pick kernel writes the forced id without
         # reading them, so those steps replay a graph WITHOUT the LM head (51290 x 768, the largest GEMM of the step).  The
         # decoder layers still run: the KV cache of the step is needed by the following steps.
-        return dict(idx=idx, r0=r0, r1=r1, ops=ops_, pick=pick, step=step, n_unf=n_unf, graph=None, graph_forced=None,
-                    stream=torch.cuda.Stream(device=self.dev), full=ops_ + [lambda: pick(None), lambda: ops.step_advance(step)],
-                    full_forced=ops_[:-1] + [lambda: pick(None), lambda: ops.step_advance(step)])
+        self.dec_full_forced = ops_[:-1] + tail
+        self.g_dec = None
+        self.g_dec_forced = None
 
     # ------------------------------------------------------------------ running
-    def _run(self, lst, holder, key, tag, replay_after_capture=True):
+    def _run(self, lst, key, tag, replay_after_capture=True):
         if not self.use_graph:
             for f in lst:
                 f()
             return
-        g = holder[key] if isinstance(holder, dict) else getattr(holder, key)
+        g = getattr(self, key)
         if g is None:
             # first use: one eager pass (lazy one-time setup must not happen inside a capture), capture, and -- unless the
             # caller keeps the eager results (B2P_EAGER_FIRST, debugging) -- the results come from replaying the graph, so
@@ -497,14 +441,11 @@ class FlorencePlan:
                 with torch.cuda.graph(g, stream=ops.capture_stream(tag, self.dev), capture_error_mode="thread_local"):
                     for f in lst:
                         f()
-            if isinstance(holder, dict):
-                holder[key] = g
-            else:
-                setattr(holder, key, g)
+            setattr(self, key, g)
             if not replay_after_capture or os.environ.get("B2P_EAGER_FIRST"):
                 return
         g.replay()
-        ops.count_graph_launches(sum(getattr(f, "n_kernels", 1) for f in lst))
+        ops.count_graph_launches(len(lst))
 
     def warm(self):
         """Build every CUDA graph of this plan on scratch inputs (call with the GPU otherwise idle: see
@@ -515,27 +456,24 @@ class FlorencePlan:
         self.encode()
         self.reset_decode(self.K)
         self.decode_step()
-        self.join()
         torch.cuda.current_stream().synchronize()
         self.warmed = True
 
     def _warm_decode(self):
-        """Capture the decode-step graph(s) on scratch state (one eager step + capture), before any real decoding."""
-        if not self.use_graph or os.environ.get("B2P_EAGER_FIRST") or all(pt["graph"] is not None and pt["graph_forced"] is not None for pt in self.parts):
+        """Capture the two decode-step graphs on scratch state (one eager step + capture each), before any real decoding."""
+        if not self.use_graph or os.environ.get("B2P_EAGER_FIRST") or (self.g_dec is not None and self.g_dec_forced is not None):
             return
         self._reset_state(self.K)
-        self.decode_step(_warm=True)
-        self.join()
-        self.decode_step(_warm=True, forced=True)     # the LM-head-free graph of the forced steps
-        self.join()
+        self.decode_step()
+        self.decode_step(forced=True)     # the LM-head-free graph of the forced steps
         torch.cuda.current_stream().synchronize()
 
     def encode(self, from_resized: bool = False):
         """from_resized: the SxS crops are already in ``crops_in`` (host-side processor did the bicubic resize)."""
         if from_resized and self.S != 64:
-            self._run(self.enc_ops[1:], self, "g_enc_nr", self.tag)
+            self._run(self.enc_ops[1:], "g_enc_nr", self.tag)
         else:
-            self._run(self.enc_ops, self, "g_enc", self.tag)
+            self._run(self.enc_ops, "g_enc", self.tag)
 
     def reset_decode(self, n_active: int):
         self._warm_decode()
@@ -547,56 +485,32 @@ class FlorencePlan:
         self.finished.zero_()
         if n_active < self.K:
             self.finished[n_active:] = 1     # padding rows never gate the stop test
-        for pt in self.parts:
-            pt["step"].zero_()
-            pt["n_unf"].fill_(max(0, min(n_active, pt["r1"]) - pt["r0"]))
-        self._forked = False
+        self.step.zero_()
+        self.n_unf.fill_(max(0, min(n_active, self.K)))
 
     def unfinished(self) -> int:
-        tot = 0
-        for pt in self.parts:
-            if len(self.parts) > 1:
-                pt["stream"].synchronize()
-            tot += int(pt["n_unf"].item())
-        return tot
+        return int(self.n_unf.item())
 
     def step_is_forced(self, t: int) -> bool:
         """True if the token of decode step t (0-based) is fixed by the generation config whatever the logits are."""
         g = self.w.gen
-        if os.environ.get("B2P_NO_FORCED_SKIP"):
-            return False
         return (t == 0 and g.get("forced_bos_token_id") is not None) or (t == self.T - 1 and g.get("forced_eos_token_id") is not None)
 
-    def decode_step(self, dump=None, force_tokens=None, _warm=False, forced=False):
+    def decode_step(self, dump=None, force_tokens=None, forced=False):
         """one token for every row; ``force_tokens`` [K] (teacher forcing) overwrites the picked ids.  forced: this step's
         token is forced by the generation config (``step_is_forced``): run the step without the LM head."""
         if dump is None and force_tokens is None:
-            cur = torch.cuda.current_stream()
-            lst, key = ("full_forced", "graph_forced") if forced else ("full", "graph")
-            if len(self.parts) == 1:
-                self._run(self.parts[0][lst], self.parts[0], key, self.tag + "_dec0", replay_after_capture=False)
-                return
-            if not self._forked:
-                for pt in self.parts:
-                    pt["stream"].wait_stream(cur)     # encoder outputs / reset are ready
-                self._forked = True
-            for pt in self.parts:
-                with torch.cuda.stream(pt["stream"]):
-                    self._run(pt[lst], pt, key, f"{self.tag}_dec{pt['idx']}", replay_after_capture=False)
+            lst, key = (self.dec_full_forced, "g_dec_forced") if forced else (self.dec_full, "g_dec")
+            self._run(lst, key, self.tag + "_dec0", replay_after_capture=False)
             return
-        for pt in self.parts:   # eager path used by the parity tests
-            for f in pt["ops"]:
-                f()
-            pt["pick"](dump[pt["r0"]:pt["r1"]] if dump is not None else None)
-            if force_tokens is not None:
-                t = int(pt["step"].item())
-                self.seq[pt["r0"]:pt["r1"], t + 1] = force_tokens[pt["r0"]:pt["r1"]]
-            ops.step_advance(pt["step"])
+        for f in self.dec_ops:   # eager path used by the parity tests
+            f()
+        self.pick(dump)
+        if force_tokens is not None:
+            t = int(self.step.item())
+            self.seq[:, t + 1] = force_tokens
+        ops.step_advance(self.step)
 
     def join(self):
-        """make the current stream wait for the decode chains (call before reading seq / starting the next encode)."""
-        if len(self.parts) > 1 and getattr(self, "_forked", False):
-            cur = torch.cuda.current_stream()
-            for pt in self.parts:
-                cur.wait_stream(pt["stream"])
-            self._forked = False
+        """No-op, kept for callers that synchronise with the decoder before reading ``seq``: the decode step runs on the
+        caller's stream, so stream order already covers it."""

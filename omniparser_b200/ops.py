@@ -101,13 +101,6 @@ def gemm(a_ptr, lda, w, M, N, K, out_ptr, ldc, bias=None, res_ptr=None, ldr=0, a
                                    flags, _stream()))
 
 
-def gemm_ln(a_ptr, lda, w, M, N, K, bias, res, ldr, gamma, beta, out16, ld16, out32, ld32, eps=1e-5, split=False, x3=False):
-    """out = LayerNorm(A @ w^T + bias + res): park-only GEMM + split-K-reduce/LayerNorm kernel (decoder out-proj / fc2)."""
-    flags = (FLAG_SPLIT if split else 0) | (FLAG_X3 if x3 else 0)
-    _lib.check(_lib.lib().b2p_gemm_ln(_p(a_ptr), lda, _p(w), M, N, K, _p(bias), _p(res), ldr, _p(gamma), _p(beta), eps,
-                                      _p(out16), ld16, _p(out32), ld32, flags, _stream()))
-
-
 def linear(x: torch.Tensor, w: torch.Tensor, bias=None, res=None, act=ACT_NONE, out_dtype=torch.float16, out=None,
            bn_max=0):
     """out[M,N] = act(x[M,K] @ w[N,K]^T + bias) + res ; x, w fp16 row-major (x may be a strided row view)."""
@@ -245,16 +238,11 @@ def layernorm(x, gamma, beta, T, C, out16=None, out32=None, eps=1e-5, split=Fals
                                         _p(out32), C, int(split), _stream()))
 
 
-def dwconv3x3_res(x, B, H, W, C, w9c, bias, y):
-    _lib.check(_lib.lib().b2p_dwconv3x3_res(_p(x), B, H, W, C, _p(w9c), _p(bias), _p(y), _stream()))
-
-
-def dwconv_ln(x, B, H, W, C, w9c, bias, y, gamma, beta, out16, eps=1e-5, split=False, tile=False, v3=False):
-    """y = dwconv3x3(x) + bias + x (fp32) and out16 = LayerNorm(y) as the next GEMM operand, one kernel.  tile: smem-tiled
-    variant (one CTA per image, maps up to 200 KB); v3: strip kernel with register-resident weights (csrc/florence_simt.cu;
-    shapes it does not cover fall back to the tile / per-token kernels)."""
+def dwconv_ln(x, B, H, W, C, w9c, bias, y, gamma, beta, out16, eps=1e-5, split=False, v3=False):
+    """y = dwconv3x3(x) + bias + x (fp32) and out16 = LayerNorm(y) as the next GEMM operand, one kernel.  v3: strip kernel
+    with register-resident weights (csrc/florence_simt.cu; shapes it does not cover fall back to the per-token kernel)."""
     _lib.check(_lib.lib().b2p_dwconv_ln(_p(x), B, H, W, C, _p(w9c), _p(bias), _p(y), _p(gamma), _p(beta), eps, _p(out16),
-                                        int(bool(split)) | (2 if tile else 0) | (4 if v3 else 0), _stream()))
+                                        int(bool(split)) | (4 if v3 else 0), _stream()))
 
 
 def window_attn(qkv32, qkv_bias, B, H, W, C, heads, out, win=12, split=False, v3=False):
@@ -263,10 +251,9 @@ def window_attn(qkv32, qkv_bias, B, H, W, C, heads, out, win=12, split=False, v3
                                           int(bool(split)) | (4 if v3 else 0), _stream()))
 
 
-def channel_attn(qkv32, B, N, C, groups, out, split=False, small=False, v3=False):
-    """small: warp-per-(batch, group) variant for N <= 16 tokens; v3: register-tiled kernel (csrc/florence_simt.cu)."""
-    _lib.check(_lib.lib().b2p_channel_attn(_p(qkv32), B, N, C, groups, _p(out),
-                                           int(bool(split)) | (2 if small else 0) | (4 if v3 else 0), _stream()))
+def channel_attn(qkv32, B, N, C, groups, out, split=False, v3=False):
+    """v3: register-tiled kernel (csrc/florence_simt.cu)."""
+    _lib.check(_lib.lib().b2p_channel_attn(_p(qkv32), B, N, C, groups, _p(out), int(bool(split)) | (4 if v3 else 0), _stream()))
 
 
 def mha(q, ldq, k, v, ldk, B, Lq, Lk, heads, out, ldo, split=False, v3=False):

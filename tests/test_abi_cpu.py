@@ -17,7 +17,7 @@ def _declared():
     return sorted(set(re.findall(r"\b(b2p_[a-z0-9_]+)\s*\(", text)))
 
 
-def test_library_builds_and_exports_every_declared_symbol():
+def test_abi3_library_builds_and_exports_every_declared_symbol():
     _lib.build()
     lib = ctypes.CDLL(str(_lib.LIB_PATH))
     names = _declared()
@@ -25,7 +25,7 @@ def test_library_builds_and_exports_every_declared_symbol():
     for n in names:
         assert hasattr(lib, n), f"{n} declared in include/b200parse.h but not exported"
     assert set(_lib.PROTOTYPES) == set(names), set(_lib.PROTOTYPES) ^ set(names)
-    assert _lib.lib().b2p_abi_version() == 2
+    assert _lib.lib().b2p_abi_version() == 3
 
 
 def test_no_libcuda_link_dependency():

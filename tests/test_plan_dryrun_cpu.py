@@ -91,7 +91,10 @@ def _check(name, a):
         assert ldx >= Cc and (o16 is None or ld16 >= (2 if split else 1) * Cc) and (o32 is None or ld32 >= Cc)
     elif name in ("b2p_dwconv_ln", "b2p_channel_attn", "b2p_window_attn", "b2p_mha", "b2p_mha_cached", "b2p_projector_prep"):
         split = a[-2]
-        assert 0 <= split <= 7            # bit 0: [hi | lo] output, bit 1: round-2 tile/small variants, bit 2: florence_simt.cu kernels
+        if name in ("b2p_dwconv_ln", "b2p_channel_attn", "b2p_window_attn", "b2p_mha"):
+            assert split in (0, 1, 4, 5)  # bit 0: [hi | lo] output, bit 2: florence_simt.cu kernels
+        else:
+            assert split in (0, 1)
 
 
 @pytest.fixture()
@@ -138,20 +141,6 @@ def test_florence_plan_64(rec, florence, prec):
     assert len(forced) == n_dec - 1 and forced[-3:] == ["b2p_layernorm", "b2p_greedy_pick", "b2p_step_advance"]
 
 
-def test_gemm_ln_opt_in(rec, florence, monkeypatch):
-    """B2P_GEMM_LN=1: the 18 (split-K GEMM + residual, LayerNorm) pairs of the decode step become b2p_gemm_ln calls"""
-    from omniparser_b200.florence_engine import FlorencePlan, FlorenceWeights
-    monkeypatch.setenv("B2P_GEMM_LN", "1")
-    w = FlorenceWeights(florence.state_dict(), torch.device("cpu"), FS.GEN, "fp16x3")
-    p = FlorencePlan(w, 2, 4, FS.PROMPT_IDS, use_graph=False, size=64)
-    p.encode()
-    n_enc = len(rec.calls)
-    p.reset_decode(2)
-    p.decode_step()
-    names = [c[0] for c in rec.calls[n_enc:]]
-    assert len(names) == 71 - 18 and names.count("b2p_gemm_ln") == 18 and names.count("b2p_layernorm") == 1
-
-
 def test_florence_plan_768(rec, florence):
     from omniparser_b200.florence_engine import FlorencePlan, FlorenceWeights
     w = FlorenceWeights(florence.state_dict(), torch.device("cpu"), FS.GEN, "fp16x3")
@@ -166,29 +155,29 @@ def test_florence_plan_768(rec, florence):
     assert len(rec.calls) == n_all - 1 and rec.calls[0][0] == "b2p_im2col_u8"
 
 
-def test_kernel_variant_flags_are_forwarded(rec, florence, monkeypatch):
+def test_simt_flags_fixed_and_retired_switches_ignored(rec, florence, monkeypatch):
+    """every SIMT entry point of the encode asks for the florence_simt.cu kernel (bit 2) and, in fp16x3 mode, for the
+    [hi | lo] output (bit 0); the environment switches of the retired kernel variants no longer change anything"""
     from omniparser_b200.florence_engine import FlorencePlan, FlorenceWeights
-    monkeypatch.delenv("B2P_NO_DWCONV_TILE", raising=False)
-    monkeypatch.delenv("B2P_NO_CHATTN_SMALL", raising=False)
-    monkeypatch.delenv("B2P_NO_SIMT_V3", raising=False)
-    w = FlorenceWeights(florence.state_dict(), torch.device("cpu"), FS.GEN, "fp16x3")
-    p = FlorencePlan(w, 2, 2, FS.PROMPT_IDS, use_graph=False, size=64)
-    p.encode()
-    assert {c[1][-2] for c in rec.calls if c[0] == "b2p_dwconv_ln"} == {7}        # default: florence_simt.cu kernels, tile / small as fall-backs
-    assert {c[1][-2] for c in rec.calls if c[0] == "b2p_channel_attn"} == {7}
-    assert {c[1][-2] for c in rec.calls if c[0] in ("b2p_window_attn", "b2p_mha")} == {5}
-    rec.calls.clear()
-    monkeypatch.setenv("B2P_NO_SIMT_V3", "1")
-    p = FlorencePlan(w, 2, 2, FS.PROMPT_IDS, use_graph=False, size=64)
-    p.encode()
-    assert {c[1][-2] for c in rec.calls if c[0] in ("b2p_dwconv_ln", "b2p_channel_attn")} == {3}   # smem-tiled / warp-per-group variants
-    assert {c[1][-2] for c in rec.calls if c[0] in ("b2p_window_attn", "b2p_mha")} == {1}
-    rec.calls.clear()
-    monkeypatch.setenv("B2P_NO_DWCONV_TILE", "1")
-    monkeypatch.setenv("B2P_NO_CHATTN_SMALL", "1")
-    p = FlorencePlan(w, 2, 2, FS.PROMPT_IDS, use_graph=False, size=64)
-    p.encode()
-    assert {c[1][-2] for c in rec.calls if c[0] in ("b2p_dwconv_ln", "b2p_channel_attn")} == {1}   # the round-1 kernels
+    retired = ("B2P_NO_SIMT_V3", "B2P_NO_DWCONV_TILE", "B2P_NO_CHATTN_SMALL", "B2P_GEMM_LN", "B2P_NO_FORCED_SKIP", "B2P_DECODE_PARTS")
+    for prec, want in (("fp16x3", 5), ("fp16", 4)):
+        w = FlorenceWeights(florence.state_dict(), torch.device("cpu"), FS.GEN, prec)
+        for env in ("", "2"):
+            for k in retired:
+                if env:
+                    monkeypatch.setenv(k, env)
+                else:
+                    monkeypatch.delenv(k, raising=False)
+            rec.calls.clear()
+            p = FlorencePlan(w, 2, 2, FS.PROMPT_IDS, use_graph=False, size=64)
+            p.encode()
+            for name in ("b2p_dwconv_ln", "b2p_window_attn", "b2p_channel_attn", "b2p_mha"):
+                assert {c[1][-2] for c in rec.calls if c[0] == name} == {want}, (name, prec, env)
+            n_enc = len(rec.calls)
+            p.reset_decode(2)
+            p.decode_step()
+            names = [c[0] for c in rec.calls[n_enc:]]
+            assert len(names) == 71 and names.count("b2p_layernorm") == 1 + 3 * 6 and p.step_is_forced(0), (prec, env)
 
 
 # ---- data flow of the pooled caption-encoder plan -------------------------------------------------------------------
@@ -295,7 +284,7 @@ class _Graph:
         _Graph.replays += 1
 
 
-def test_graph_paths(rec, florence, monkeypatch):
+def test_graph_paths_single_decode_chain(rec, florence, monkeypatch):
     """first-use capture, warm(), replay bookkeeping (CUDA graphs replaced by a stub that counts replays)"""
     from omniparser_b200.florence_engine import FlorencePlan, FlorenceWeights
     from omniparser_b200.yolo_engine import YoloPlan, YoloWeights
@@ -309,7 +298,7 @@ def test_graph_paths(rec, florence, monkeypatch):
     p = FlorencePlan(w, 2, 3, FS.PROMPT_IDS, use_graph=True, size=64)
     assert p.use_graph and not p.warmed
     p.warm()                                            # encode: eager + capture + replay; decode: eager + capture, then one replay
-    assert p.warmed and p.g_enc is not None and all(pt["graph"] is not None and pt["graph_forced"] is not None for pt in p.parts)
+    assert p.warmed and p.g_enc is not None and p.g_dec is not None and p.g_dec_forced is not None
     n_eager = len(rec.calls)
     assert n_eager == 2 * (232 + 71 + 70)               # every op ran once eagerly and once inside the (stubbed) capture; the
                                                         # decode step exists with and without the LM head (forced tokens)

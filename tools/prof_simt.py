@@ -42,9 +42,9 @@ def mh(v3):
     labels.append(f"mha L=13 v3={v3}")
 
 
-dw(4, 512, v3=True); dw(4, 512, tile=True); dw(16, 128, v3=True); dw(16, 128, tile=True); dw(16, 128)
+dw(4, 512, v3=True); dw(16, 128, v3=True); dw(16, 128)
 wa(4, 512, 16, True); wa(4, 512, 16, False); wa(8, 256, 8, True)
-ca(16, 512, v3=True); ca(16, 512, small=True); ca(256, 128, v3=True); ca(256, 128)
+ca(16, 512, v3=True); ca(256, 128, v3=True); ca(256, 128)
 mh(True); mh(False)
 x = ops.new_map(8, 160, 160, 256, DEV); x.buf.normal_()
 x1 = ops.new_map(8, 160, 160, 128, DEV); x2 = ops.new_map(8, 80, 80, 128, DEV)

@@ -30,7 +30,7 @@ def _wrap(name):
     return w
 
 
-for n in ("gemm", "gemm_ln", "conv1x1", "conv3x3", "adown_pool", "maxpool_s1", "upsample2x", "im2col3x3", "cbfuse", "im2col_u8", "layernorm",
+for n in ("gemm", "conv1x1", "conv3x3", "adown_pool", "maxpool_s1", "upsample2x", "im2col3x3", "cbfuse", "im2col_u8", "layernorm",
           "dwconv_ln", "window_attn", "channel_attn", "mha", "mha_cached", "encoder_embed", "decoder_embed", "projector_prep",
           "greedy_pick", "step_advance", "resize_u8"):
     setattr(ops, n, _wrap(n))
@@ -79,7 +79,7 @@ if what in ("florence", "all"):
     plan.decode_step()
     torch.cuda.synchronize()
     time_ops(plan.enc_ops, "enc")
-    time_ops(plan.parts[0]["ops"] + [lambda: plan.parts[0]["pick"](None)], "dec")
+    time_ops(plan.dec_ops + [lambda: plan.pick(None)], "dec")
 
 if what in ("yolo", "all"):
     from omniparser_b200.yolo_engine import YoloPlan, YoloWeights
